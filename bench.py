@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — Lanczos e^A·x throughput on B200 (BASELINE.json metric: Lanczos iterations/s + SpMV GB/s vs HBM roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3] [--impl reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P bench.py --gpus N ...
 
 One "step" = one full e^A·x evaluation on the workload graph: k Lanczos steps (fused SpMV+alpha, fused update+norm,
@@ -227,6 +227,26 @@ def make_csr_file(w, scale_override, n_override, path, device):
     return n, nnz
 
 
+DUMP_SAMPLE = 1 << 21   # entries of e^A x that --dump-outputs writes at most: 16 MB of values + 16 MB of vertex ids
+
+
+def dump_outputs(ctx, out_dir, write):
+    """--dump-outputs: what a caller of the timed step receives, e^A x (lz_get_ans) and the tridiagonal (lz_get_tridiag), as
+    float64 .npy files. Above DUMP_SAMPLE vertices ans.npy is a fixed seeded sample and ans_index.npy holds its vertex ids.
+    Collective on several GPUs (lz_get_ans gathers the vector); only a rank with `write` set touches the file system."""
+    y = ctx.get_ans()
+    alpha, beta = ctx.get_tridiag()
+    if not write:
+        return
+    os.makedirs(out_dir, exist_ok=True)
+    out = {"alpha": alpha, "beta": beta, "ans": y}
+    if len(y) > DUMP_SAMPLE:
+        idx = np.sort(np.random.default_rng(20261018).choice(len(y), DUMP_SAMPLE, replace=False))
+        out["ans"], out["ans_index"] = y[idx], idx.astype(np.float64)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def sample_iters_for(nnz):
     # ~1e-8 s per stored entry per CPU iteration at large n (measured: 108 ms/iter at nnz 1.68e7) -> aim for ~10-15 s
     per_iter = max(nnz * 1.2e-8, 1e-4)
@@ -247,7 +267,11 @@ def main():
     ap.add_argument("--no-reorth-detail", action="store_true")
     ap.add_argument("--no-f32-detail", action="store_true")
     ap.add_argument("--save-summary", default=None, help="write a summary fixture (.npz) of this run's answer (rank 0)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the last step's e^A x (sampled on large graphs) and alpha/beta as DIR/*.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the answer of --impl ours")
 
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -361,6 +385,8 @@ def main():
     launches = tm.kernel_launches - launches0
     ms = max_over_ranks(ms)
     value = k * args.steps / (ms * 1e-3)
+    if args.dump_outputs:
+        dump_outputs(ctx, args.dump_outputs, rank == 0)
     if graph_replay:
         ctx.set_profiling(True)
         step(); ctx.sync(); step(); ctx.sync()

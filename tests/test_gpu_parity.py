@@ -528,3 +528,22 @@ def test_reorth_second_pass_path(always):
     assert out["second_passes"] == (29 if always == "1" else out["second_passes"])
     if always == "0":
         assert out["second_passes"] <= 29
+
+
+def test_bench_dump_outputs_match_reference_golden(lz, orc, golden, tmp_path):
+    """bench.py --dump-outputs on C1 (the graph of c1_er_n10000_k20) writes the last timed step's e^A x and tridiagonal: the
+    reference's answer to the same tolerances as above, next to the usual result line."""
+    import json
+    import os
+    import subprocess
+    import sys
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "c1", "--steps", "2", "--warmup", "1",
+                        "--no-cpu-baseline", "--no-f32-detail", "--dump-outputs", str(tmp_path)], capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    assert json.loads(r.stdout.strip().splitlines()[-1])["steps"] == 2
+    g = golden("c1_er_n10000_k20")
+    y, alpha, beta = (np.load(tmp_path / f"{f}.npy") for f in ("ans", "alpha", "beta"))
+    assert rel2(y, g["ans"]) < TOL and np.array_equal(orc.top_k(y), orc.top_k(g["ans"]))
+    np.testing.assert_allclose(alpha[:6], g["alpha"][:6], rtol=1e-8)
+    np.testing.assert_allclose(beta[:5], g["beta"][:5], rtol=1e-8)

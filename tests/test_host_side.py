@@ -182,3 +182,38 @@ def test_bench_step_breakdown_parses_a_device_timeline():
     assert out["spmv_pass0_wait_for_chunk"] == 1.0 and out["spmv_pass0_gather"] == 100.0 and out["spmv_pass0_senders_next_chunk"] == 90.0
     assert out["spmv_pass1_wait_for_chunk"] == 2.0 and out["spmv_pass1_senders_next_chunk"] is None
     assert out["wait_total_max_over_ranks"] == 12.0
+
+
+def test_bench_dump_outputs_writes_float_arrays_and_a_fixed_sample(tmp_path):
+    """bench.dump_outputs (--dump-outputs): float64 .npy files of the answer and the tridiagonal; a vector longer than
+    DUMP_SAMPLE becomes the same seeded sample on every run, with its vertex ids; a rank without `write` writes nothing."""
+    sys.path.insert(0, ROOT)
+    import bench
+
+    class FakeCtx:
+        def __init__(self, n):
+            self.y = np.random.default_rng(n).random(n)
+
+        def get_ans(self):
+            return self.y
+
+        def get_tridiag(self):
+            return np.arange(1.0, 6.0), np.arange(1.0, 5.0)
+    small, big = FakeCtx(1000), FakeCtx(bench.DUMP_SAMPLE + 12345)
+    bench.dump_outputs(small, str(tmp_path / "small"), True)
+    assert sorted(os.listdir(tmp_path / "small")) == ["alpha.npy", "ans.npy", "beta.npy"]
+    assert np.array_equal(np.load(tmp_path / "small" / "ans.npy"), small.y)
+    runs = []
+    for d in ("big1", "big2"):
+        bench.dump_outputs(big, str(tmp_path / d), True)
+        runs.append({f: np.load(tmp_path / d / f) for f in os.listdir(tmp_path / d)})
+    assert sorted(runs[0]) == ["alpha.npy", "ans.npy", "ans_index.npy", "beta.npy"]
+    assert all(a.dtype == np.float64 for a in runs[0].values())
+    assert all(np.array_equal(runs[0][f], runs[1][f]) for f in runs[0])
+    idx = runs[0]["ans_index.npy"].astype(np.int64)
+    assert len(idx) == bench.DUMP_SAMPLE and np.all(np.diff(idx) > 0) and idx[-1] < len(big.y)
+    assert np.array_equal(runs[0]["ans.npy"], big.y[idx])
+    assert np.array_equal(runs[0]["alpha.npy"], np.arange(1.0, 6.0))
+    assert sum(os.path.getsize(tmp_path / "big1" / f) for f in runs[0]) <= 64 << 20
+    bench.dump_outputs(big, str(tmp_path / "other_rank"), False)
+    assert not os.path.exists(tmp_path / "other_rank")

@@ -234,8 +234,10 @@ def test_oracle_analytic_eigen_combination(lz, orc):
     n, ro, ci = lz.generate_host(lz.GraphSpec.er(1500, 6000, 17))
     x, y = analytic_eigen_combination(ro, ci)
     rel = {}
-    for k in (5, 20, 30, 45):
+    for k in (5, 10, 20, 30, 45):
         ans, _, _ = orc.expv(ro, ci, k, x)
         rel[k] = np.linalg.norm(ans - y) / np.linalg.norm(y)
-    assert rel[5] > 1e-3 and rel[20] < 1e-6 and rel[30] < 1e-10 and rel[45] < 1e-11, rel
-    assert rel[5] > rel[20] > rel[30]
+    assert rel[5] > 1e-3 and 1e-8 < rel[10] < 1e-4 and rel[20] < 1e-11 and rel[30] < 1e-10 and rel[45] < 1e-11, rel
+    # from k = 20 on the error sits at rounding level (5e-15 .. 1e-14, depending on the host's LAPACK), where the order of
+    # two k's is noise: past that point a larger k may only stay at that level
+    assert rel[5] > rel[10] > rel[20] and rel[30] <= max(rel[20], 1e-14), rel
