@@ -138,13 +138,35 @@ int lz_lanczos_run(lz_ctx* ctx, uint32_t k, int reorth);
 /* alpha[k], beta[k-1] to the host (cu_lanczos.cu:129-130). Synchronises. Either pointer may be NULL. */
 int lz_get_tridiag(lz_ctx* ctx, double* alpha_out, double* beta_out);
 /* On-device eigendecomposition of T = tridiag(beta, alpha, beta) and coefficient vector
- *   c = ||x|| * Z * (exp(lambda) .* Z^T e1)
+ *   c = ||x|| * Z * (f(lambda) .* Z^T e1),   f = exp by default (see lz_set_matfun)
  * Replaces eigenDecomp<T> (LAPACKE_dstevd, parallel-final/lib/eigen.cu:17-21) + multiplyOut.cu:30-40. Enqueue only. */
 int lz_tridiag_expv(lz_ctx* ctx);
+/* Matrix function applied by the coefficient solve, so that lz_multout yields f(A) x. Ritz values theta_j, parameter p:
+ *   LZ_MATFUN_EXP        exp(p*theta)            e^{pA} x: total communicability at inverse temperature p. (EXP, 1.0) is the
+ *                                                default and gives the same bits as a context that never calls this.
+ *   LZ_MATFUN_EXP_SCALED exp(p*theta - ls)       e^{p(A - sI)} x with s the Ritz value maximising p*theta and ls = p*s, so
+ *                                                e^{pA} x = ans * e^ls. Never overflows (plain EXP fails with LZ_ERR_NUMERIC once
+ *                                                p*theta_max passes ~709); ls is on the device, read it with lz_get_matfun_scale.
+ *   LZ_MATFUN_RESOLVENT  1 / (1 - p*theta)       (I - pA)^{-1} x; with x = ones this is Katz centrality (up to subtracting x,
+ *                                                which leaves the ranking unchanged). LZ_ERR_NUMERIC with its own message when
+ *                                                1 - p*theta_j <= 0 for some Ritz value. That check sees theta_max <= lambda_max
+ *                                                only: passing it does not prove p < 1/lambda_max. The Ritz values of any graph
+ *                                                (theta_max among them) come from EXP_SCALED followed by lz_get_eigen.
+ * Followed by lz_tridiag_expv, lz_get_eigen (coefficients), lz_estimate_change, lz_choose_k, lz_expv_host(_root); lz_multout,
+ * lz_get_ans and lz_top_k consume the coefficients as before. Drops the coefficients and the answer but keeps the tridiagonal and
+ * the basis, so one lz_lanczos_run serves any number of functions. Kept across start vectors and runs. LZ_ERR_ARG for an unknown
+ * kind or a non-finite parameter. With world > 1 every rank must pass the same values (every rank then computes the same c). */
+#define LZ_MATFUN_EXP 0
+#define LZ_MATFUN_EXP_SCALED 1
+#define LZ_MATFUN_RESOLVENT 2
+int lz_set_matfun(lz_ctx* ctx, int kind, double param);
+/* log of the factor the last lz_tridiag_expv left out: ls = p*s under LZ_MATFUN_EXP_SCALED, 0 otherwise. Synchronises.
+ * LZ_ERR_ARG before lz_tridiag_expv. */
+int lz_get_matfun_scale(lz_ctx* ctx, double* log_scale_out);
 /* Optional read-back: eigenvalues ascending [k], eigenvectors row-major [k*k] with eigvecs[i*k+j] = component i of
  * vector j (the LAPACK_ROW_MAJOR layout eigen.cu:20 produces), coeff [k]. Synchronises. Any pointer may be NULL. */
 int lz_get_eigen(lz_ctx* ctx, double* eigvals_out, double* eigvecs_out, double* coeff_out);
-/* Convergence estimate: relative 2-norm change of e^A x between Krylov dimensions k_prev < k (k = the last run), from the
+/* Convergence estimate: relative 2-norm change of e^A x (f(A) x, lz_set_matfun) between Krylov dimensions k_prev < k (k = the last run), from the
  * tridiagonal alone (no pass over the basis). The reference has no such check; its author recommends one (writeup sec. 11). */
 int lz_estimate_change(lz_ctx* ctx, uint32_t k_prev, double* rel_out);
 /* The smallest Krylov dimension k' <= k (k = the last run) such that every dimension in [k', k] reproduces the k-step answer to

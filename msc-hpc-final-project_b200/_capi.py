@@ -20,6 +20,7 @@ REORTH_NONE, REORTH_FULL = 0, 1
 EXCHANGE_NONE, EXCHANGE_NCCL, EXCHANGE_PEER_DENSE, EXCHANGE_PEER_SPARSE = 0, 1, 2, 3
 SPMV_AUTO, SPMV_VECTOR, SPMV_WARP = 0, 1, 2
 BASIS_F64, BASIS_F32 = 0, 1
+MATFUN_EXP, MATFUN_EXP_SCALED, MATFUN_RESOLVENT = 0, 1, 2
 NCCL_UID_BYTES = 128
 
 
@@ -106,6 +107,8 @@ _sig("lz_spmv_host", _ctx, _f64p, _f64p)
 _sig("lz_get_basis", _ctx, C.c_uint32, _f64p)
 _sig("lz_set_spmv_variant", _ctx, C.c_int)
 _sig("lz_set_basis_precision", _ctx, C.c_int)
+_sig("lz_set_matfun", _ctx, C.c_int, C.c_double)
+_sig("lz_get_matfun_scale", _ctx, _P(C.c_double))
 _sig("lz_set_profiling", _ctx, C.c_int)
 _sig("lz_exchange_info", _ctx, _P(C.c_int), _P(C.c_double))
 _sig("lz_timings_get", _ctx, _P(Timings))
@@ -339,6 +342,17 @@ class Context:
 
     def set_basis_precision(self, p):
         _check(lib.lz_set_basis_precision(self._h, p))
+
+    def set_matfun(self, kind, param):
+        """kind: MATFUN_EXP (e^{pA} x), MATFUN_EXP_SCALED (e^{p(A - sI)} x, see matfun_scale) or MATFUN_RESOLVENT
+        ((I - pA)^{-1} x, Katz centrality). Keeps the last Lanczos run: tridiag_expv + multout apply the new function."""
+        _check(lib.lz_set_matfun(self._h, kind, param))
+
+    def matfun_scale(self):
+        """log of the factor the last tridiag_expv left out: f(A) x = answer * exp(matfun_scale())."""
+        r = C.c_double(0)
+        _check(lib.lz_get_matfun_scale(self._h, C.byref(r)))
+        return r.value
 
     def set_spmv_variant(self, v):
         _check(lib.lz_set_spmv_variant(self._h, v))

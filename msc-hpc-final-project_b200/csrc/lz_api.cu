@@ -451,6 +451,30 @@ extern "C" int lz_set_basis_precision(lz_ctx* c, int precision) {
   return LZ_OK;
 }
 
+static const char* const kIndefiniteMsg =
+    "resolvent: 1 - alpha * theta <= 0 for a Ritz value theta, (I - alpha A) is not positive definite (alpha >= 1 / lambda_max)";
+
+// Only the coefficient solve depends on the function: the tridiagonal and the basis stay valid, the coefficients and the answer go.
+extern "C" int lz_set_matfun(lz_ctx* c, int kind, double param) {
+  if (!c) return lz_fail(LZ_ERR_ARG, "null ctx");
+  if (kind != LZ_MATFUN_EXP && kind != LZ_MATFUN_EXP_SCALED && kind != LZ_MATFUN_RESOLVENT)
+    return lz_fail(LZ_ERR_ARG, "unknown matrix function %d", kind);
+  if (!isfinite(param)) return lz_fail(LZ_ERR_ARG, "matrix function parameter must be finite");
+  c->matfun_kind = kind;
+  c->matfun_param = param;
+  c->have_coef = c->have_ans = false;
+  return LZ_OK;
+}
+
+extern "C" int lz_get_matfun_scale(lz_ctx* c, double* log_scale_out) {
+  if (!c || !log_scale_out) return lz_fail(LZ_ERR_ARG, "null argument");
+  if (!c->have_coef) return lz_fail(LZ_ERR_ARG, "lz_tridiag_expv must be called before lz_get_matfun_scale");
+  LZ_TRY(set_dev(c));
+  LZ_CUDA(cudaMemcpyAsync(log_scale_out, c->scal + 5, 8, cudaMemcpyDeviceToHost, c->stream));
+  LZ_CUDA(cudaStreamSynchronize(c->stream));
+  return LZ_OK;
+}
+
 extern "C" int lz_set_spmv_variant(lz_ctx* c, int variant) {
   if (!c || variant < 0 || variant > LZ_SPMV_WARP) return lz_fail(LZ_ERR_ARG, "bad SpMV variant");
   c->spmv_variant = variant;
@@ -755,6 +779,7 @@ extern "C" int lz_get_eigen(lz_ctx* c, double* eigvals_out, double* eigvecs_out,
   LZ_CUDA(cudaMemcpyAsync(&st, c->status, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
   LZ_CUDA(cudaStreamSynchronize(c->stream));
   if (st & 0x3FFFFFFF) return lz_fail(LZ_ERR_NUMERIC, "tridiagonal eigensolver: eigenvalue %d did not converge", (st & 0x3FFFFFFF) - 1);
+  if (st & kStatusIndefinite) return lz_fail(LZ_ERR_NUMERIC, kIndefiniteMsg);
   if (st & 0x40000000) return lz_fail(LZ_ERR_NUMERIC, "coefficient vector is not finite (exp of a Ritz value overflowed, or breakdown)");
   return LZ_OK;
 }
@@ -763,26 +788,29 @@ extern "C" int lz_get_eigen(lz_ctx* c, double* eigvals_out, double* eigvecs_out,
 // || y_k - y_k' ||_2 = || c_k - [c_k'; 0] ||_2, so the change of the answer between Krylov dimensions k' < k costs two
 // k x k eigen-solves and no pass over the basis.
 namespace {
+// Under LZ_MATFUN_EXP_SCALED every block uses the shift of the full k x k solve (which runs first), so all c_k' carry the same
+// factor e^{-ls} and the relative change is the unscaled one; by interlacing no leading block has a larger t*theta.
 struct CoefSolver {   // scratch for solves of leading blocks of the current tridiagonal; nothing of the ctx's result is touched
   lz_ctx* c;
   uint32_t k;
-  double *ev = nullptr, *evec = nullptr, *work = nullptr, *coef = nullptr;
+  double *ev = nullptr, *evec = nullptr, *work = nullptr, *coef = nullptr, *ls = nullptr;
   int* st = nullptr;
   CoefSolver(lz_ctx* c_, uint32_t k_) : c(c_), k(k_) {}
-  ~CoefSolver() { cudaFree(ev); cudaFree(evec); cudaFree(work); cudaFree(coef); cudaFree(st); }
+  ~CoefSolver() { cudaFree(ev); cudaFree(evec); cudaFree(work); cudaFree(coef); cudaFree(ls); cudaFree(st); }
   int init() {
     LZ_CUDA(cudaMalloc((void**)&ev, k * 8)); LZ_CUDA(cudaMalloc((void**)&evec, (size_t)k * k * 8));
     LZ_CUDA(cudaMalloc((void**)&work, (size_t)k * k * 8)); LZ_CUDA(cudaMalloc((void**)&coef, k * 8));
-    LZ_CUDA(cudaMalloc((void**)&st, sizeof(int)));
+    LZ_CUDA(cudaMalloc((void**)&ls, 8)); LZ_CUDA(cudaMalloc((void**)&st, sizeof(int)));
     return LZ_OK;
   }
-  int solve(uint32_t kk, std::vector<double>& out) {   // out = c_kk (kk entries)
+  int solve(uint32_t kk, std::vector<double>& out) {   // out = c_kk (kk entries); solve(k) first
     out.assign(kk, 0.0);
     int sth = 0;
-    LZ_TRY(lz_k_tridiag_expv_into(c, kk, ev, evec, work, coef, st));
+    LZ_TRY(lz_k_tridiag_expv_into(c, kk, ev, evec, work, coef, st, kk == k ? nullptr : ls, kk == k ? ls : nullptr));
     LZ_CUDA(cudaMemcpyAsync(out.data(), coef, kk * 8, cudaMemcpyDeviceToHost, c->stream));
     LZ_CUDA(cudaMemcpyAsync(&sth, st, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
     LZ_CUDA(cudaStreamSynchronize(c->stream));
+    if (sth & kStatusIndefinite) return lz_fail(LZ_ERR_NUMERIC, kIndefiniteMsg);
     if (sth) return lz_fail(LZ_ERR_NUMERIC, "tridiagonal solve of the leading %u x %u block failed or overflowed (status %d)", kk, kk, sth);
     return LZ_OK;
   }
@@ -901,6 +929,7 @@ static int expv_impl(lz_ctx* c, const double* x_host, uint32_t k, int reorth, do
   int st = 0;
   LZ_CUDA(cudaMemcpy(&st, c->status, sizeof(int), cudaMemcpyDeviceToHost));
   if (st & 0x3FFFFFFF) return lz_fail(LZ_ERR_NUMERIC, "tridiagonal eigensolver: eigenvalue %d did not converge", (st & 0x3FFFFFFF) - 1);
+  if (st & kStatusIndefinite) return lz_fail(LZ_ERR_NUMERIC, kIndefiniteMsg);
   if (st & 0x40000000) return lz_fail(LZ_ERR_NUMERIC, "result is not finite (exp of a Ritz value overflowed, or Lanczos breakdown)");
   return LZ_OK;
 }

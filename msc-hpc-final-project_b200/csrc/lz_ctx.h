@@ -151,7 +151,8 @@ struct lz_ctx {
   bool lagged = true;              // use the lagged normalisation where it applies (one GPU, no reorthogonalisation); LZ_LAGGED_NORM=0 disables
   bool lagged_done = false;        // the last run left rows 1.. of V unnormalised
   bool lagged_run = false;         // set by the step loop that is being enqueued
-  double* scal = nullptr;          // device scalars: [0]=alpha acc, [1]=norm2 acc, [2]=x_norm, [3..] spare
+  double* scal = nullptr;          // device scalars: [0]=alpha acc, [1]=norm2 acc, [2]=x_norm, [5]=log scale of the last
+                                   // coefficient solve (lz_get_matfun_scale), others: scratch of the step loop and set-up
   double* partials = nullptr;      // device, per-CTA partial sums
   uint32_t partials_cap = 0;
   unsigned int* ticket = nullptr;  // device, last-block counters
@@ -161,6 +162,8 @@ struct lz_ctx {
   double* eigwork = nullptr;
   double* coef = nullptr;          // device, [k_cap]
   int* status = nullptr;           // device: [0] eigensolver status, [1] reorth skip flag, [2] second-pass counter
+  int matfun_kind = LZ_MATFUN_EXP; // function the coefficient solve applies (lz_set_matfun); kept across runs and start vectors
+  double matfun_param = 1.0;
   bool have_x = false, have_tridiag = false, have_coef = false, have_ans = false;
   void* flush_buf = nullptr;
   size_t flush_bytes = 0;
@@ -237,8 +240,13 @@ int lz_k_combine(lz_ctx* c, const void* V, bool f32, uint32_t nvec, const double
                  double* norm2_out /* device scalar or null */, const int* skip = nullptr, float* out32 = nullptr /* fp32 copy of out */);
 int lz_k_reorth_decide(lz_ctx* c, const double* norm2_before, const double* norm2_after, int* skip, unsigned int* second_passes);
 int lz_k_reorth_select(lz_ctx* c, const int* skip, const double* norm2_second, double* norm2, double* norm2_copy = nullptr, double* beta_out = nullptr);
-int lz_k_tridiag_expv(lz_ctx* c, uint32_t k);
-int lz_k_tridiag_expv_into(lz_ctx* c, uint32_t k, double* eigvals, double* eigvecs, double* work, double* coef, int* status);
+// eigensolver status word: bits 0-29 = 1 + index of an eigenvalue that did not converge, bit 30 = coefficients not finite,
+// bit 31 = resolvent denominator 1 - alpha*theta <= 0 for some Ritz value theta
+constexpr int kStatusIndefinite = (int)0x80000000u;
+int lz_k_tridiag_expv(lz_ctx* c, uint32_t k);   // the ctx's result; log scale -> scal[5]
+// ls_in: shift to use for LZ_MATFUN_EXP_SCALED instead of the block's own (null: own); ls_out (may be null) receives the one used
+int lz_k_tridiag_expv_into(lz_ctx* c, uint32_t k, double* eigvals, double* eigvecs, double* work, double* coef, int* status,
+                           const double* ls_in, double* ls_out);
 // dst[i] = x_orig[new2old[first + i]] (/ sqrt(*norm2) when norm2 != null), i < count; padding slots -> 0
 int lz_k_permute_in(lz_ctx* c, const double* x_orig, const double* norm2, uint64_t first, uint64_t count, double* dst);
 int lz_k_permute_out(lz_ctx* c, const double* y_new_full, double* y_orig);

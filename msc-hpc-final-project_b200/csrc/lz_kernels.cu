@@ -1208,18 +1208,25 @@ __global__ void __launch_bounds__(kBlock) k_combine(const TV* __restrict__ V, ui
 // One CTA. Thread 0 runs the scalar implicit-shift QL recurrences and publishes each sweep's rotations; all threads apply
 // them to the eigenvector matrix, kept transposed (zt[i*k + q] = component q of vector i) so the update is coalesced.
 // Output in the layout LAPACKE_dstevd(LAPACK_ROW_MAJOR,'V') gives the reference (eigen.cu:20): eigenvalues ascending,
-// eigvecs[q*k + j] = component q of eigenvector j. Then f_j = exp(lambda_j) * x_norm * eigvecs[0*k + j] (multiplyOut.cu:30-33)
-// and coef = eigvecs * f (multiplyOut.cu:40).
+// eigvecs[q*k + j] = component q of eigenvector j. Then f_j = f(lambda_j) * x_norm * eigvecs[0*k + j] (multiplyOut.cu:30-33)
+// and coef = eigvecs * f (multiplyOut.cu:40), with f selected by fkind (LZ_MATFUN_*):
+//   EXP        exp(p*lambda - 0)   (p = 1: exactly the reference's exp(lambda))
+//   EXP_SCALED exp(p*lambda - ls), ls = max_j p*lambda_j, or *ls_in when given (leading blocks reuse the full solve's shift);
+//              every argument is <= 0, so nothing overflows for any graph
+//   RESOLVENT  1 / (1 - p*lambda); a non-positive denominator sets kStatusIndefinite
+// ls goes to *ls_out (when given) so that e^{pA} x = ans * e^ls.
 constexpr int kEigMax = 1024;
 __global__ void __launch_bounds__(kBlock) k_tridiag_expv(uint32_t k, const double* __restrict__ alpha, const double* __restrict__ beta,
                                                          const double* __restrict__ xnorm2_p, double* __restrict__ eigvals,
                                                          double* __restrict__ eigvecs, double* __restrict__ zt_global, double* __restrict__ coef,
-                                                         int* __restrict__ status, int zt_in_smem) {
+                                                         int* __restrict__ status, int zt_in_smem, int fkind, double fparam,
+                                                         const double* __restrict__ ls_in, double* __restrict__ ls_out) {
   extern __shared__ double zt_smem[];
   double* zt = zt_in_smem ? zt_smem : zt_global;   // k*k doubles: shared memory when it fits (k <= ~150), else global scratch
   __shared__ double d[kEigMax], e[kEigMax], cs[kEigMax], sn[kEigMax];
   __shared__ int perm[kEigMax];
   __shared__ int s_m, s_sweep, s_cont, s_fail;
+  __shared__ double s_ls;
   const int n = (int)k, tid = threadIdx.x;
   for (int i = tid; i < n; i += kBlock) {
     d[i] = alpha[i];
@@ -1326,9 +1333,33 @@ __global__ void __launch_bounds__(kBlock) k_tridiag_expv(uint32_t k, const doubl
     const int q = i / n, j = i % n;
     eigvecs[i] = zt[perm[j] * n + q];
   }
+  if (tid == 0) {
+    double ls = 0.0;
+    if (fkind == LZ_MATFUN_EXP_SCALED) {
+      if (ls_in) ls = *ls_in;
+      else {
+        ls = -INFINITY;
+        for (int j = 0; j < n; j++) ls = fmax(ls, fparam * d[j]);   // NaNs (breakdown) are skipped here and poison f below
+      }
+    }
+    s_ls = ls;
+    if (ls_out) *ls_out = ls;
+  }
   __syncthreads();
-  const double xn = sqrt(*xnorm2_p);
-  for (int j = tid; j < n; j += kBlock) cs[j] = exp(d[perm[j]]) * xn * eigvecs[j];   // f_j ; row 0 of eigvecs
+  const double xn = sqrt(*xnorm2_p), ls = s_ls;
+  bool indefinite = false;
+  for (int j = tid; j < n; j += kBlock) {   // f_j ; row 0 of eigvecs
+    const double lam = d[perm[j]];
+    double fj;
+    if (fkind == LZ_MATFUN_RESOLVENT) {
+      const double den = 1.0 - fparam * lam;
+      indefinite |= den <= 0.0;
+      fj = 1.0 / den;
+    } else {
+      fj = exp(fparam * lam - ls);
+    }
+    cs[j] = fj * xn * eigvecs[j];
+  }
   __syncthreads();
   bool bad = false;
   for (int i = tid; i < n; i += kBlock) {
@@ -1340,6 +1371,7 @@ __global__ void __launch_bounds__(kBlock) k_tridiag_expv(uint32_t k, const doubl
   if (tid == 0) *status = s_fail;
   __syncthreads();
   if (bad) atomicOr(status, 0x40000000);
+  if (indefinite) atomicOr(status, kStatusIndefinite);
 }
 
 // "Twice is enough" (Daniel-Gragg-Kaufman-Stewart): after one classical Gram-Schmidt pass the second is needed only if the
@@ -1611,25 +1643,20 @@ int lz_k_reorth_select(lz_ctx* c, const int* skip, const double* norm2_second, d
 }
 
 // Same solve for the leading k x k block into caller-provided scratch (convergence estimate; nothing of the ctx's result is touched).
-int lz_k_tridiag_expv_into(lz_ctx* c, uint32_t k, double* eigvals, double* eigvecs, double* work, double* coef, int* status) {
+int lz_k_tridiag_expv_into(lz_ctx* c, uint32_t k, double* eigvals, double* eigvecs, double* work, double* coef, int* status,
+                           const double* ls_in, double* ls_out) {
   if (k > (uint32_t)kEigMax) return lz_fail(LZ_ERR_ARG, "krylov dimension %u exceeds the on-device eigensolver limit %d", k, kEigMax);
   const size_t zt_bytes = (size_t)k * k * sizeof(double);
   const int in_smem = zt_bytes <= 180 * 1024;
   if (in_smem) LZ_CUDA(cudaFuncSetAttribute(k_tridiag_expv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)zt_bytes));
-  k_tridiag_expv<<<1, kBlock, in_smem ? zt_bytes : 0, c->stream>>>(k, c->alpha, c->beta, c->scal + 2, eigvals, eigvecs, work, coef, status, in_smem);
+  k_tridiag_expv<<<1, kBlock, in_smem ? zt_bytes : 0, c->stream>>>(k, c->alpha, c->beta, c->scal + 2, eigvals, eigvecs, work, coef, status, in_smem,
+                                                                  c->matfun_kind, c->matfun_param, ls_in, ls_out);
   LZ_LAUNCH_CHECK();
   return LZ_OK;
 }
 
 int lz_k_tridiag_expv(lz_ctx* c, uint32_t k) {
-  if (k > (uint32_t)kEigMax) return lz_fail(LZ_ERR_ARG, "krylov dimension %u exceeds the on-device eigensolver limit %d", k, kEigMax);
-  const size_t zt_bytes = (size_t)k * k * sizeof(double);
-  const int in_smem = zt_bytes <= 180 * 1024;
-  if (in_smem) LZ_CUDA(cudaFuncSetAttribute(k_tridiag_expv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)zt_bytes));
-  k_tridiag_expv<<<1, kBlock, in_smem ? zt_bytes : 0, c->stream>>>(k, c->alpha, c->beta, c->scal + 2, c->eigvals, c->eigvecs, c->eigwork,
-                                                                  c->coef, c->status, in_smem);
-  LZ_LAUNCH_CHECK();
-  return LZ_OK;
+  return lz_k_tridiag_expv_into(c, k, c->eigvals, c->eigvecs, c->eigwork, c->coef, c->status, nullptr, c->scal + 5);
 }
 
 int lz_k_permute_in(lz_ctx* c, const double* x_orig, const double* norm2, uint64_t first, uint64_t count, double* dst) {

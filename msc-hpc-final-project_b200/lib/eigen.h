@@ -2,6 +2,8 @@
 // The reference calls LAPACKE_dstevd on the host; here the k x k tridiagonal is solved on the device (lz_tridiag_expv),
 // together with the coefficient vector multOut needs. eigenvalues are ascending; eigenvectors[i*k + j] = component i of
 // eigenvector j — the layout LAPACK_ROW_MAJOR dstevd returns. Unlike the reference, L.beta is left intact.
+// eigenDecomp(L, kind, param) first selects the matrix function multOut applies (lz_set_matfun: LZ_MATFUN_EXP with inverse
+// temperature param, LZ_MATFUN_EXP_SCALED, LZ_MATFUN_RESOLVENT for Katz); the one-argument form keeps e^A.
 #ifndef LZ_EIGEN_H
 #define LZ_EIGEN_H
 
@@ -24,6 +26,11 @@ class eigenDecomp {
       : eigenvalues(new T[_L.krylov_dim]), eigenvectors(new T[(size_t)_L.krylov_dim * _L.krylov_dim]), L{_L} {
     decompose();
   }
+  eigenDecomp(lanczosDecomp<T>& _L, int kind, double param)
+      : eigenvalues(new T[_L.krylov_dim]), eigenvectors(new T[(size_t)_L.krylov_dim * _L.krylov_dim]), L{_L} {
+    if (lz_set_matfun(L.ctx, kind, param) != LZ_OK) lanczosDecomp<T>::fail("eigenDecomp: lz_set_matfun");
+    decompose();
+  }
   eigenDecomp(eigenDecomp<T>&) = delete;
   eigenDecomp& operator=(eigenDecomp<T>&) = delete;
   ~eigenDecomp() {
@@ -32,6 +39,12 @@ class eigenDecomp {
   }
   const T* get_eigenvalues() const { return eigenvalues; }
   const T* get_eigenvectors() const { return eigenvectors; }
+  // f(A) x = ans * e^log_scale(): nonzero only for LZ_MATFUN_EXP_SCALED
+  double log_scale() const {
+    double ls = 0.0;
+    if (lz_get_matfun_scale(L.ctx, &ls) != LZ_OK) lanczosDecomp<T>::fail("eigenDecomp: lz_get_matfun_scale");
+    return ls;
+  }
   template <typename U> friend void multOut(lanczosDecomp<U>&, eigenDecomp<U>&, adjMatrix&, bool);
 };
 

@@ -8,6 +8,8 @@
 //   options: --reorth (full reorthogonalisation)  --gpus N (row-sharded, one host thread per GPU, NCCL)
 //            --check FILE (raw float64 e^A x to compare with, e.g. written by oracle/_ref/ref_final --out)
 //            --write FILE (one value per line, write_ans)   --top M (print the M most central vertices, device-side ranking)
+//            --t T (e^{TA} x, inverse temperature T)   --scaled (e^{T(A - sI)} x, s = largest Ritz value: never overflows; the log
+//            scale T*s is printed)   --katz ALPHA ((I - ALPHA A)^{-1} x, Katz centrality)
 //
 // Same object sequence as the reference: adjMatrix -> lanczosDecomp<double>(A,k,x,cuda=true) -> eigenDecomp<double> ->
 // multOut(L,E,A,true), same TIMING / ERROR CHECKING tables. The reference's serial arm (main.cu:83-99) is not here: this
@@ -35,7 +37,8 @@
 static double seconds_between(timeval s, timeval e) { return e.tv_sec - s.tv_sec + (e.tv_usec - s.tv_usec) / 1000000.0; }
 
 // Row-sharded run over `gpus` devices: one host thread per GPU, each driving its own lz_ctx (C ABI directly).
-static int run_multi(adjMatrix& A, unsigned k, int reorth, int gpus, std::vector<double>& ans, double& t_lanczos, double& t_mult) {
+static int run_multi(adjMatrix& A, unsigned k, int reorth, int gpus, int fkind, double fparam, std::vector<double>& ans, double& log_scale,
+                     double& t_lanczos, double& t_mult) {
   unsigned char uid[LZ_NCCL_UID_BYTES];
   if (lz_nccl_unique_id(uid) != LZ_OK) { std::cerr << lz_last_error() << '\n'; return 1; }
   std::vector<int> rc(gpus, 0);
@@ -48,6 +51,7 @@ static int run_multi(adjMatrix& A, unsigned k, int reorth, int gpus, std::vector
       auto bad = [&](int code) { rc[r] = code; err[r] = lz_last_error(); if (c) lz_destroy(c); };
       int e;
       if ((e = lz_create_dist(r, r, gpus, uid, &c)) != LZ_OK) return bad(e);
+      if ((e = lz_set_matfun(c, fkind, fparam)) != LZ_OK) return bad(e);
       if ((e = lz_csr_upload(c, A.get_n(), A.get_row_offset(), A.get_col_idx())) != LZ_OK) return bad(e);
       if ((e = lz_set_start_vector(c, nullptr)) != LZ_OK) return bad(e);
       if ((e = lz_sync(c)) != LZ_OK) return bad(e);
@@ -62,7 +66,10 @@ static int run_multi(adjMatrix& A, unsigned k, int reorth, int gpus, std::vector
       if ((e = lz_get_ans(c, y.data())) != LZ_OK) return bad(e);
       gettimeofday(&e2, NULL);
       tl[r] = seconds_between(s, e1); tm[r] = seconds_between(e1, e2);
-      if (r == 0) ans.swap(y);
+      if (r == 0) {
+        if ((e = lz_get_matfun_scale(c, &log_scale)) != LZ_OK) return bad(e);
+        ans.swap(y);
+      }
       lz_destroy(c);
     });
   }
@@ -82,12 +89,21 @@ int main(int argc, char** argv) {
   uint64_t seed = 1;
   int reorth = LZ_REORTH_NONE, gpus = 1;
   unsigned top = 0;
+  double t = 1.0, katz = 0.0;
+  bool scaled = false, have_t = false, have_katz = false;
 
   // long options first; what is left goes to the reference's getopt string
   std::vector<char*> rest{argv[0]};
   for (int i = 1; i < argc; i++) {
     std::string a = argv[i];
     auto val = [&]() -> const char* { if (i + 1 >= argc) { std::cerr << "missing value for " << a << '\n'; exit(2); } return argv[++i]; };
+    auto num = [&]() -> double {
+      const char* v = val();
+      char* end = nullptr;
+      const double d = strtod(v, &end);
+      if (end == v || *end) { std::cerr << "not a number for " << a << ": " << v << '\n'; exit(2); }
+      return d;
+    };
     if (a == "--graph") graph = val();
     else if (a == "--scale") scale = (unsigned)atoi(val());
     else if (a == "--ef") ef = (unsigned)atoi(val());
@@ -98,9 +114,19 @@ int main(int argc, char** argv) {
     else if (a == "--gpus") gpus = atoi(val());
     else if (a == "--reorth") reorth = LZ_REORTH_FULL;
     else if (a == "--top") top = (unsigned)atoi(val());
+    else if (a == "--t") { t = num(); have_t = true; }
+    else if (a == "--scaled") scaled = true;
+    else if (a == "--katz") { katz = num(); have_katz = true; }
     else rest.push_back(argv[i]);
   }
   if (parseArguments((int)rest.size(), rest.data(), filename, krylov_dim, verbose, n, deg, edges) != 0) return 2;
+  if (have_katz && (have_t || scaled)) { std::cerr << "--katz excludes --t and --scaled\n"; return 2; }
+  const int fkind = have_katz ? LZ_MATFUN_RESOLVENT : scaled ? LZ_MATFUN_EXP_SCALED : LZ_MATFUN_EXP;
+  const double fparam = have_katz ? katz : t;
+  const bool default_fun = fkind == LZ_MATFUN_EXP && fparam == 1.0;
+  std::string fun_label = "total communicability";
+  if (have_katz) fun_label = "Katz centrality (I - alpha A)^-1 x, alpha = " + std::to_string(fparam);
+  else if (!default_fun) fun_label = "total communicability e^{tA} x, t = " + std::to_string(fparam) + (scaled ? ", scaled by e^-log_scale" : "");
 
   timeval start, end;
   gettimeofday(&start, NULL);
@@ -139,17 +165,17 @@ int main(int argc, char** argv) {
 
   std::vector<double> x_double(n, 1);   // main.cu:79
   std::vector<double> result;
-  double gpu_time_lanczos = 0, gpu_time_mult = 0, gpu_time_whole = 0;
+  double gpu_time_lanczos = 0, gpu_time_mult = 0, gpu_time_whole = 0, log_scale = 0;
   lz_timings tm{};
   if (gpus > 1) {
-    if (run_multi(A, krylov_dim, reorth, gpus, result, gpu_time_lanczos, gpu_time_mult)) return 1;
+    if (run_multi(A, krylov_dim, reorth, gpus, fkind, fparam, result, log_scale, gpu_time_lanczos, gpu_time_mult)) return 1;
     gpu_time_whole = gpu_time_lanczos + gpu_time_mult;
   } else {
     timeval s, e1, e2, e3;
     gettimeofday(&s, NULL);
     lanczosDecomp<double> cu_L(A, krylov_dim, &x_double[0], /*cuda=*/true, reorth);   // main.cu:115
     gettimeofday(&e1, NULL);
-    eigenDecomp<double> cu_E(cu_L);                                                   // main.cu:124
+    eigenDecomp<double> cu_E(cu_L, fkind, fparam);                                    // main.cu:124
     gettimeofday(&e2, NULL);
     multOut(cu_L, cu_E, A, true);                                                     // main.cu:127
     gettimeofday(&e3, NULL);
@@ -158,17 +184,21 @@ int main(int argc, char** argv) {
     gpu_time_whole = seconds_between(s, e3);
     tm = cu_L.timings();
     result.assign(cu_L.get_ans_ptr(), cu_L.get_ans_ptr() + n);
+    log_scale = cu_E.log_scale();
     if (!write_file.empty()) write_ans(write_file, cu_L);                             // main.cu:159
     if (top) {
       std::vector<unsigned> ti(top);
       std::vector<double> tv(top);
       const unsigned cnt = cu_L.top_k(top, ti.data(), tv.data());
-      std::cout << "TOP " << cnt << " vertices by total communicability (rank vertex value)\n" << std::setprecision(17);
+      std::cout << "TOP " << cnt << " vertices by " << fun_label << " (rank vertex value)\n" << std::setprecision(17);
       for (unsigned i = 0; i < cnt; i++) std::cout << "rank " << i + 1 << ' ' << ti[i] << ' ' << tv[i] << '\n';
       std::cout << std::setprecision(6);
     }
   }
 
+  if (!default_fun)
+    std::cout << "matrix function: " << fun_label << "\nlog scale: " << std::setprecision(17) << log_scale << std::setprecision(6)
+              << " (f(A) x = result * e^log_scale)\n";
   std::cout << std::setfill('~') << std::setw(WIDTH) << '\n' << std::setfill(' ');
   std::cout << "TIMING (host wall clock, seconds; Lanczos includes CSR upload and relabelling as the reference's includes its cudaMalloc + H2D)\n";
   std::cout << std::setfill('~') << std::setw(WIDTH) << '\n' << std::setfill(' ');
