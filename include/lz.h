@@ -186,6 +186,35 @@ int lz_get_ans(lz_ctx* ctx, double* ans_host);
  * *count_out (optional) = min(m, n) valid pairs. Synchronises. With world > 1 the call is collective and every rank receives the
  * same result (idx_out / val_out may be NULL on ranks that do not need it). */
 int lz_top_k(lz_ctx* ctx, uint32_t m, uint32_t* idx_out, double* val_out, uint32_t* count_out);
+/* ---- top Ritz pairs: eigenvector centrality and a certified spectral-radius bracket ----------------------------------------------
+ * After lz_lanczos_run(k) let T = Z Theta Z^T (Theta ascending). For j = 0..m-1: theta_j is the j-th largest Ritz value and
+ * y_j = V z_j / ||V z_j|| its Ritz vector, unit 2-norm, sign chosen so that sum_i y_j(i) >= 0. Then, with a real SpMV,
+ *   rho_j = y_j^T A y_j             the Rayleigh quotient,
+ *   r_j   = ||A y_j - rho_j y_j||_2 the true residual (not the Lanczos estimate beta_k |e_k^T z_j|, which needs the beta_k the run does not
+ *                                   compute and is not valid once orthogonality is lost).
+ * A is symmetric, so [rho_j - r_j, rho_j + r_j] contains an eigenvalue of A (Krylov-Bogoliubov) for plain and reorthogonalised runs,
+ * fp64 or fp32 basis, lagged or not. A plain run can return two copies of a converged eigenvalue when m > 1 ("ghosts"); each interval
+ * is still correct. Use LZ_REORTH_FULL and a random start vector when the pairs beyond the first matter.
+ * Spectral-radius bracket lo <= lambda_max <= hi, for every graph (connected or not): lo = rho_0; hi = max_i (A z)_i / z_i over the
+ * vertices (Collatz-Wielandt, A >= 0, z > 0) with z_i = max(|y_0(i)|, LZ_CW_FLOOR * max|y_0|), inflated by the fp64 rounding
+ * allowance (max_degree + 2) * 2^-52 (relative). Tight when y_0 has converged on a connected graph. hi certifies a Katz parameter:
+ * alpha = f / hi with f < 1 gives alpha < 1 / lambda_max.
+ *
+ * lz_ritz: 1 <= m <= min(LZ_RITZ_MAX, k). Collective when world > 1; synchronises once at the end. Leaves y_0 as the answer, so
+ * lz_get_ans / lz_top_k return eigenvector centrality (lz_multout brings f(A) x back). Does not touch the coefficients, the
+ * tridiagonal or the basis. Works after a coefficient solve that overflowed (only the eigensolver's convergence is checked).
+ * LZ_ERR_ARG: bad m or no run. LZ_ERR_NUMERIC: eigensolver failure, a zero Ritz vector or non-finite results.
+ * A new run, start vector, graph or basis precision drops the pairs; lz_set_matfun keeps them. */
+#define LZ_RITZ_MAX 16
+#define LZ_CW_FLOOR 1e-6
+int lz_ritz(lz_ctx* ctx, uint32_t m);
+/* m values each, largest first. Any pointer may be NULL. LZ_ERR_ARG before lz_ritz. */
+int lz_get_ritz(lz_ctx* ctx, double* theta_out, double* rayleigh_out, double* resid_out);
+/* y_j (n doubles, original vertex order), j < m. Collective when world > 1; NULL on ranks that do not need the vector. */
+int lz_get_ritz_vector(lz_ctx* ctx, uint32_t j, double* y_host);
+/* lo <= lambda_max <= hi (see above); identical on every rank. LZ_ERR_ARG before lz_ritz. */
+int lz_spectral_radius_bounds(lz_ctx* ctx, double* lo_out, double* hi_out);
+
 /* Whole pipeline with HOST buffers, what lanczosDecomp<double>(A,k,x,true) + eigenDecomp + multOut do in main.cu:115-127:
  * H2D x, k steps, eigensolve, multOut, D2H ans. */
 int lz_expv_host(lz_ctx* ctx, const double* x_host, uint32_t k, int reorth, double* ans_host);

@@ -13,5 +13,5 @@ from ._capi import (  # noqa: F401
     write_bin, csr_from_edges, device_count, nccl_unique_id, exported_symbols, header_symbols,
     GRAPH_ER, GRAPH_RMAT, GRAPH_BAND, REORTH_NONE, REORTH_FULL, SPMV_AUTO, SPMV_VECTOR, SPMV_WARP,
     EXCHANGE_NONE, EXCHANGE_NCCL, EXCHANGE_PEER_DENSE, EXCHANGE_PEER_SPARSE, BASIS_F64, BASIS_F32,
-    MATFUN_EXP, MATFUN_EXP_SCALED, MATFUN_RESOLVENT,
+    MATFUN_EXP, MATFUN_EXP_SCALED, MATFUN_RESOLVENT, RITZ_MAX, CW_FLOOR,
 )

@@ -21,6 +21,8 @@ EXCHANGE_NONE, EXCHANGE_NCCL, EXCHANGE_PEER_DENSE, EXCHANGE_PEER_SPARSE = 0, 1, 
 SPMV_AUTO, SPMV_VECTOR, SPMV_WARP = 0, 1, 2
 BASIS_F64, BASIS_F32 = 0, 1
 MATFUN_EXP, MATFUN_EXP_SCALED, MATFUN_RESOLVENT = 0, 1, 2
+RITZ_MAX = 16
+CW_FLOOR = 1e-6
 NCCL_UID_BYTES = 128
 
 
@@ -109,6 +111,10 @@ _sig("lz_set_spmv_variant", _ctx, C.c_int)
 _sig("lz_set_basis_precision", _ctx, C.c_int)
 _sig("lz_set_matfun", _ctx, C.c_int, C.c_double)
 _sig("lz_get_matfun_scale", _ctx, _P(C.c_double))
+_sig("lz_ritz", _ctx, C.c_uint32)
+_sig("lz_get_ritz", _ctx, _f64p, _f64p, _f64p)
+_sig("lz_get_ritz_vector", _ctx, C.c_uint32, _f64p)
+_sig("lz_spectral_radius_bounds", _ctx, _P(C.c_double), _P(C.c_double))
 _sig("lz_set_profiling", _ctx, C.c_int)
 _sig("lz_exchange_info", _ctx, _P(C.c_int), _P(C.c_double))
 _sig("lz_timings_get", _ctx, _P(Timings))
@@ -353,6 +359,29 @@ class Context:
         r = C.c_double(0)
         _check(lib.lz_get_matfun_scale(self._h, C.byref(r)))
         return r.value
+
+    def ritz(self, m):
+        """Top m Ritz pairs of the last Lanczos run -> (theta, rayleigh, resid), largest first. [rayleigh - resid, rayleigh + resid]
+        contains an eigenvalue of A. Leaves y_0 (eigenvector centrality) as the answer: get_ans / top_k read it."""
+        _check(lib.lz_ritz(self._h, m))
+        th, rho, res = np.empty(m), np.empty(m), np.empty(m)
+        _check(lib.lz_get_ritz(self._h, _f64(th), _f64(rho), _f64(res)))
+        return th, rho, res
+
+    def ritz_vector(self, j, want_result=True):
+        """y_j in original vertex order (unit 2-norm, non-negative sum). want_result=False (world > 1 only): take part only."""
+        if not want_result:
+            _check(lib.lz_get_ritz_vector(self._h, j, None))
+            return None
+        y = np.empty(self.graph_info().n)
+        _check(lib.lz_get_ritz_vector(self._h, j, _f64(y)))
+        return y
+
+    def spectral_radius_bounds(self):
+        """(lo, hi) with lo <= lambda_max <= hi, after ritz()."""
+        lo, hi = C.c_double(0), C.c_double(0)
+        _check(lib.lz_spectral_radius_bounds(self._h, C.byref(lo), C.byref(hi)))
+        return lo.value, hi.value
 
     def set_spmv_variant(self, v):
         _check(lib.lz_set_spmv_variant(self._h, v))

@@ -90,6 +90,7 @@ void free_vectors(lz_ctx* c) {
   c->V = c->w = c->xfull = c->xstage = c->ans = c->alpha = c->beta = c->hcoef = c->eigvals = c->eigvecs = c->eigwork = c->coef = nullptr;
   c->k_cap = 0;
   c->have_x = c->have_tridiag = c->have_coef = c->have_ans = false;
+  cudaFree(c->ritz_R); c->ritz_R = nullptr; c->ritz_rows = 0; c->ritz_m = 0;
 }
 
 // Peer exchange set-up (collective: every rank calls it at the same point). Each rank publishes CUDA IPC handles of its
@@ -734,6 +735,7 @@ extern "C" int lz_lanczos_run(lz_ctx* c, uint32_t k, int reorth) {
   if (!done) LZ_TRY(enqueue_steps(c, k, reorth, fused_push, peer_scalars));
   LZ_CUDA(cudaEventRecord(c->ev_b, c->stream));
   c->k_done = k;
+  c->run_serial++;
   c->lagged_done = c->lagged_run;
   c->reorth_done = reorth;
   c->have_tridiag = true;
@@ -909,6 +911,132 @@ extern "C" int lz_get_ans(lz_ctx* c, double* ans_host) {
   if (!c->have_ans) return lz_fail(LZ_ERR_ARG, "lz_multout must be called before lz_get_ans");
   LZ_TRY(set_dev(c));
   return gather_to_host(c, c->ans, ans_host);
+}
+
+// ---- top Ritz pairs -----------------------------------------------------------------------------------------------------
+static bool ritz_valid(const lz_ctx* c) { return c->have_tridiag && c->ritz_m && c->ritz_run == c->run_serial; }
+
+// Ritz pairs of the last run, checked against A itself: a k x k solve into scratch (the ctx's coefficients stay as they are), one
+// pass over the basis for all m vectors, then per vector an SpMV for the Rayleigh quotient and a combine for the true residual.
+// The Collatz-Wielandt SpMV on weights built from y_0 bounds lambda_max from above. Outside the Lanczos loop, so the scalars of
+// several GPUs are joined with NCCL.
+extern "C" int lz_ritz(lz_ctx* c, uint32_t m) {
+  if (!c) return lz_fail(LZ_ERR_ARG, "null ctx");
+  if (!c->have_tridiag) return lz_fail(LZ_ERR_ARG, "lz_lanczos_run must be called before lz_ritz");
+  const uint32_t k = c->k_done;
+  if (m < 1 || m > LZ_RITZ_MAX || m > k) return lz_fail(LZ_ERR_ARG, "lz_ritz: m = %u must be in [1, min(%d, k = %u)]", m, LZ_RITZ_MAX, k);
+  LZ_TRY(set_dev(c));
+  c->ritz_m = 0;
+  c->have_ans = false;   // ans receives y_0
+  const uint32_t M = m == 1 ? 1 : m <= 2 ? 2 : m <= 4 ? 4 : m <= 8 ? 8 : 16;
+  if (c->ritz_rows < M) {
+    LZ_CUDA(cudaStreamSynchronize(c->stream));
+    cudaFree(c->ritz_R); c->ritz_R = nullptr; c->ritz_rows = 0;
+    if (cudaMalloc((void**)&c->ritz_R, (size_t)M * c->ldv * 8) != cudaSuccess) {
+      cudaGetLastError();
+      return lz_fail(LZ_ERR_ALLOC, "cannot allocate %u Ritz vectors of %llu doubles", M, (unsigned long long)c->ldv);
+    }
+    c->ritz_rows = M;
+  }
+  CoefSolver sv(c, k);
+  LZ_TRY(sv.init());
+  // scalars [0,16) ||y_j||^2, [16,32) sum y_j, [32,48) theta, [48,64) rho, [64,80) r^2, [80] max|y_0|, [81] Collatz-Wielandt max,
+  // [82] unused dot; then W [k][16] and the combine's per-CTA partials
+  struct Scratch { double* p = nullptr; ~Scratch() { cudaFree(p); } } aux;
+  const size_t n_part = (size_t)2 * LZ_RITZ_MAX * 8 * c->sm_count;
+  LZ_CUDA(cudaMalloc((void**)&aux.p, (96 + (size_t)k * LZ_RITZ_MAX + n_part) * 8));
+  double* s = aux.p;
+  double *nrm2 = s, *vsum = s + 16, *theta = s + 32, *rho = s + 48, *r2 = s + 64, *W = s + 96, *part = W + (size_t)k * LZ_RITZ_MAX;
+  auto* absmax = reinterpret_cast<unsigned long long*>(s + 80);
+  auto* cwmax = reinterpret_cast<unsigned long long*>(s + 81);
+  LZ_CUDA(cudaMemsetAsync(s, 0, 96 * 8, c->stream));
+  LZ_TRY(lz_k_tridiag_expv_into(c, k, sv.ev, sv.evec, sv.work, sv.coef, sv.st, nullptr, nullptr));
+  LZ_TRY(lz_k_ritz_select(c, k, m, M, sv.ev, sv.evec, c->lagged_done ? c->norm2v : nullptr, W, theta));
+  double* R = c->ritz_R;
+  if (M == 1) {
+    LZ_TRY(lz_k_combine(c, basis_ptr(c), c->basis_f32, k, W, 1.0, nullptr, R, nrm2));
+    LZ_TRY(lz_k_vsum(c, R, c->n_loc, part, vsum));
+  } else {
+    LZ_TRY(lz_k_ritz_combine(c, basis_ptr(c), c->basis_f32, k, M, W, R, part, nrm2, vsum));
+  }
+  LZ_TRY(allreduce_sum(c, s, 32));
+  LZ_TRY(lz_k_ritz_scale(c, R, m, nrm2, vsum, absmax));
+  if (c->world > 1) LZ_NCCL(lz_nccl()->AllReduce(s + 80, s + 80, 1, ncclDouble, ncclMax, c->comm, c->stream));
+  // with several GPUs the SpMV reads the gathered vector: gfull, not xfull (a faster peer may already push its next q_0 there);
+  // one GPU has no gathered vector and xfull is free for the Collatz-Wielandt weights
+  double* zfull = c->world > 1 ? c->gfull : c->xfull;
+  for (uint32_t j = 0; j < m; j++) {
+    const double* y = R + (uint64_t)j * c->ldv;
+    const double* yg = y;
+    if (c->world > 1) {
+      LZ_TRY(lz_k_spread(c, y, c->gfull));
+      LZ_TRY(allgather_chunks(c, c->gfull, false));
+      yg = c->gfull;
+    }
+    LZ_TRY(lz_k_spmv_dot(c, yg, y, c->w, rho + j));                                   // w = A y_j, rho_j = y_j . w
+    LZ_TRY(allreduce_sum(c, rho + j, 1));
+    LZ_TRY(lz_k_combine(c, y, false, 1, rho + j, -1.0, c->w, c->w, r2 + j));          // ||A y_j - rho_j y_j||^2
+    LZ_TRY(allreduce_sum(c, r2 + j, 1));
+    if (j == 0) {                                                                     // lambda_max <= max_i (A z)_i / z_i
+      LZ_TRY(lz_k_cw_z(c, yg, zfull, c->n_loc * (uint64_t)c->world, s + 80, LZ_CW_FLOOR));
+      LZ_TRY(lz_k_spmv_dot(c, zfull, y, c->w, s + 82));
+      LZ_TRY(lz_k_cw_bound(c, c->w, zfull, cwmax));
+      if (c->world > 1) LZ_NCCL(lz_nccl()->AllReduce(s + 81, s + 81, 1, ncclDouble, ncclMax, c->comm, c->stream));
+    }
+  }
+  LZ_CUDA(cudaMemcpyAsync(c->ans, R, c->n_loc * 8, cudaMemcpyDeviceToDevice, c->stream));
+  double h[82];
+  int st = 0;
+  LZ_CUDA(cudaMemcpyAsync(h, s, sizeof(h), cudaMemcpyDeviceToHost, c->stream));
+  LZ_CUDA(cudaMemcpyAsync(&st, sv.st, sizeof(int), cudaMemcpyDeviceToHost, c->stream));
+  LZ_CUDA(cudaStreamSynchronize(c->stream));
+  // bits 30 and 31 belong to the matrix function (overflow, indefinite resolvent): the eigenpairs do not depend on them
+  if (st & 0x3FFFFFFF) return lz_fail(LZ_ERR_NUMERIC, "tridiagonal eigensolver: eigenvalue %d did not converge", (st & 0x3FFFFFFF) - 1);
+  for (uint32_t j = 0; j < m; j++) {
+    if (!(h[j] > 0.0) || !isfinite(h[j])) return lz_fail(LZ_ERR_NUMERIC, "Ritz vector %u is zero or not finite (||V z||^2 = %g)", j, h[j]);
+    if (!isfinite(h[32 + j]) || !isfinite(h[48 + j]) || !isfinite(h[64 + j]))
+      return lz_fail(LZ_ERR_NUMERIC, "Ritz pair %u is not finite (theta %g, rho %g, r^2 %g)", j, h[32 + j], h[48 + j], h[64 + j]);
+    c->ritz_theta[j] = h[32 + j];
+    c->ritz_rho[j] = h[48 + j];
+    c->ritz_res[j] = sqrt(h[64 + j]);
+  }
+  // (A z)_i is a sum of deg_i exact products: computed ratio >= true ratio * (1 - (deg_i + 1) 2^-53); the allowance covers it and the
+  // rounding of the product below
+  const double cw = h[81];
+  if (!isfinite(cw)) return lz_fail(LZ_ERR_NUMERIC, "Collatz-Wielandt bound is not finite");
+  c->ritz_lo = c->ritz_rho[0];
+  c->ritz_hi = cw * (1.0 + ((double)c->max_degree + 2.0) * 0x1p-52);
+  c->ritz_m = m;
+  c->ritz_run = c->run_serial;
+  c->have_ans = true;
+  return LZ_OK;
+}
+
+extern "C" int lz_get_ritz(lz_ctx* c, double* theta_out, double* rayleigh_out, double* resid_out) {
+  if (!c) return lz_fail(LZ_ERR_ARG, "null ctx");
+  if (!ritz_valid(c)) return lz_fail(LZ_ERR_ARG, "lz_ritz must be called after the last lz_lanczos_run");
+  for (uint32_t j = 0; j < c->ritz_m; j++) {
+    if (theta_out) theta_out[j] = c->ritz_theta[j];
+    if (rayleigh_out) rayleigh_out[j] = c->ritz_rho[j];
+    if (resid_out) resid_out[j] = c->ritz_res[j];
+  }
+  return LZ_OK;
+}
+
+extern "C" int lz_get_ritz_vector(lz_ctx* c, uint32_t j, double* y_host) {
+  if (!c || (!y_host && c->world == 1)) return lz_fail(LZ_ERR_ARG, "null argument");
+  if (!ritz_valid(c)) return lz_fail(LZ_ERR_ARG, "lz_ritz must be called after the last lz_lanczos_run");
+  if (j >= c->ritz_m) return lz_fail(LZ_ERR_ARG, "Ritz vector %u not available (%u computed)", j, c->ritz_m);
+  LZ_TRY(set_dev(c));
+  return gather_to_host(c, c->ritz_R + (uint64_t)j * c->ldv, y_host);
+}
+
+extern "C" int lz_spectral_radius_bounds(lz_ctx* c, double* lo_out, double* hi_out) {
+  if (!c || !lo_out || !hi_out) return lz_fail(LZ_ERR_ARG, "null argument");
+  if (!ritz_valid(c)) return lz_fail(LZ_ERR_ARG, "lz_ritz must be called after the last lz_lanczos_run");
+  *lo_out = c->ritz_lo;
+  *hi_out = c->ritz_hi;
+  return LZ_OK;
 }
 
 static int expv_impl(lz_ctx* c, const double* x_host, uint32_t k, int reorth, double* ans_host, int root);

@@ -165,6 +165,12 @@ struct lz_ctx {
   int matfun_kind = LZ_MATFUN_EXP; // function the coefficient solve applies (lz_set_matfun); kept across runs and start vectors
   double matfun_param = 1.0;
   bool have_x = false, have_tridiag = false, have_coef = false, have_ans = false;
+  // top Ritz pairs of the run numbered ritz_run (lz_ritz): valid while have_tridiag && ritz_run == run_serial, so anything that drops
+  // the run (new run, start vector, graph, basis precision) drops them too
+  uint64_t run_serial = 0, ritz_run = 0;
+  uint32_t ritz_m = 0, ritz_rows = 0;   // pairs held; rows allocated in R
+  double* ritz_R = nullptr;             // device, [ritz_rows][ldv]: y_j, this rank's rows
+  double ritz_theta[16] = {}, ritz_rho[16] = {}, ritz_res[16] = {}, ritz_lo = 0.0, ritz_hi = 0.0;
   void* flush_buf = nullptr;
   size_t flush_bytes = 0;
 
@@ -252,3 +258,18 @@ int lz_k_permute_in(lz_ctx* c, const double* x_orig, const double* norm2, uint64
 int lz_k_permute_out(lz_ctx* c, const double* y_new_full, double* y_orig);
 int lz_k_fill(lz_ctx* c, double* p, uint64_t n, double value);
 int lz_k_reserve_partials(lz_ctx* c, uint64_t count);
+// top Ritz pairs (lz_ritz). partials: caller scratch of 2 * 16 * 8 * sm_count doubles (the loop's c->partials is baked into its CUDA
+// graph and must not be regrown here).
+// theta[j] = eigvals[k-1-j], W[t*M + j] = eigvecs[t*k + k-1-j] / (norm2 ? sqrt(norm2[t]) : 1) for j < m, 0 for m <= j < M
+int lz_k_ritz_select(lz_ctx* c, uint32_t k, uint32_t m, uint32_t M, const double* eigvals, const double* eigvecs, const double* norm2, double* W,
+                     double* theta);
+// Y[j][0..n_loc) = sum_t W[t*M + j] V[t] for j < M (M = 2, 4, 8, 16), rows of Y ldv apart; ||y_j||^2 -> nrm2[j], sum_i y_j(i) -> vsum[j]
+int lz_k_ritz_combine(lz_ctx* c, const void* V, bool f32, uint32_t k, uint32_t M, const double* W, double* Y, double* partials, double* nrm2,
+                      double* vsum);
+int lz_k_vsum(lz_ctx* c, const double* v, uint64_t n, double* partials, double* out);
+// y_j *= sgn(vsum[j]) / sqrt(nrm2[j]), j < m; max |y_0| -> *absmax0 (bit pattern of a double; zero it first)
+int lz_k_ritz_scale(lz_ctx* c, double* Y, uint32_t m, const double* nrm2, const double* vsum, unsigned long long* absmax0);
+// z[i] = max(|y[i]|, delta * *absmax), i < n
+int lz_k_cw_z(lz_ctx* c, const double* y, double* z, uint64_t n, const double* absmax, double delta);
+// *out = max(*out, max over this rank's vertices of az[l] / zfull[slot(l)]) (bit pattern of a non-negative double)
+int lz_k_cw_bound(lz_ctx* c, const double* az, const double* zfull, unsigned long long* out);

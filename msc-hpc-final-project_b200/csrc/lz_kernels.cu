@@ -1391,6 +1391,180 @@ __global__ void k_reorth_select(const int* __restrict__ skip, const double* __re
   if (beta_out) *beta_out = sqrt(*norm2);
 }
 
+// ------------------------------------------------------------------------------------------------- top Ritz pairs (lz_ritz)
+// One CTA. From the ascending solve of T: theta[j] = eigvals[k-1-j] and W[t*M + j] = s_t * eigvecs[t*k + k-1-j] for j < m, 0 for
+// m <= j < M, with s_t = 1/||u_t|| when the basis rows are unnormalised (norm2 != null: the fold k_coef_scale does), else 1.
+__global__ void k_ritz_select(uint32_t k, uint32_t m, uint32_t M, const double* __restrict__ eigvals, const double* __restrict__ eigvecs,
+                              const double* __restrict__ norm2, double* __restrict__ W, double* __restrict__ theta) {
+  for (uint32_t i = threadIdx.x; i < k * M; i += blockDim.x) {
+    const uint32_t t = i / M, j = i % M;
+    double w = 0.0;
+    if (j < m) {
+      w = eigvecs[(uint64_t)t * k + (k - 1 - j)];
+      if (norm2) w /= sqrt(norm2[t]);
+    }
+    W[i] = w;
+  }
+  for (uint32_t j = threadIdx.x; j < m; j += blockDim.x) theta[j] = eigvals[k - 1 - j];
+}
+
+// Y[j][i] = sum_t W[t][j] V[t][i] for j < M: every basis row is read once for all M Ritz vectors. Same 16-byte groups and the same
+// t-ordered fma chain per output as k_combine (so column j equals k_combine(coef = W[:, j]) bit for bit). Shared memory holds W
+// (k*M doubles, at most kEigMax * 16 * 8 = 128 KB) and each thread's running ||y_j||^2 and sum_i y_j(i) in a private column
+// (2*M*kBlock doubles; in registers they would cost 4*M of them and spill the fp32 M = 16 instance). Per-vector partials in a fixed
+// slot per CTA, summed in index order by the last CTA -> nrm2[j], vsum[j].
+template <class TV, int M>
+__global__ void __launch_bounds__(kBlock) k_ritz_combine(const TV* __restrict__ V, uint64_t ldv, uint32_t k, const double* __restrict__ W,
+                                                         double* __restrict__ Y, uint64_t n, double* partials /* [2M][grid] */,
+                                                         unsigned int* ticket, double* nrm2, double* vsum) {
+  constexpr int E = ept<TV>::value;
+  constexpr int U = M <= 4 ? 8 : (M == 8 ? 4 : 2);   // basis loads in flight per thread, traded against M*E accumulators
+  extern __shared__ double s_dyn[];
+  double* s_acc = s_dyn;                              // [2M][kBlock]: ||y_j||^2 at 2j, sum y_j at 2j + 1
+  double* s_w = s_dyn + 2 * M * kBlock;               // [k][M]
+  __shared__ bool s_last;
+  const int tid = threadIdx.x;
+  for (uint32_t i = tid; i < k * M; i += kBlock) s_w[i] = W[i];
+#pragma unroll
+  for (int v = 0; v < 2 * M; v++) s_acc[v * kBlock + tid] = 0.0;
+  __syncthreads();
+  const uint64_t ng = n / E, ldg = ldv / E;
+  for (uint64_t i = (uint64_t)blockIdx.x * kBlock + tid; i < ng; i += (uint64_t)gridDim.x * kBlock) {
+    double acc[M][E];
+#pragma unroll
+    for (int j = 0; j < M; j++)
+#pragma unroll
+      for (int e = 0; e < E; e++) acc[j][e] = 0.0;
+    uint32_t t = 0;
+    for (; t + U <= k; t += U) {
+      double vv[U][E];
+#pragma unroll
+      for (int u = 0; u < U; u++) ld_group<TV>(V, (uint64_t)(t + u) * ldg + i, vv[u]);
+#pragma unroll
+      for (int u = 0; u < U; u++)
+#pragma unroll
+        for (int j = 0; j < M; j++) {
+          const double w = s_w[(t + u) * M + j];
+#pragma unroll
+          for (int e = 0; e < E; e++) acc[j][e] += w * vv[u][e];
+        }
+    }
+    for (; t < k; t++) {
+      double vv[E];
+      ld_group<TV>(V, (uint64_t)t * ldg + i, vv);
+#pragma unroll
+      for (int j = 0; j < M; j++)
+#pragma unroll
+        for (int e = 0; e < E; e++) acc[j][e] += s_w[t * M + j] * vv[e];
+    }
+#pragma unroll
+    for (int j = 0; j < M; j++) {
+      double2* y2 = reinterpret_cast<double2*>(Y + (uint64_t)j * ldv);
+      double q = 0.0, sm = 0.0;
+#pragma unroll
+      for (int h = 0; h < E / 2; h++) y2[i * (E / 2) + h] = make_double2(acc[j][2 * h], acc[j][2 * h + 1]);
+#pragma unroll
+      for (int e = 0; e < E; e++) { q += acc[j][e] * acc[j][e]; sm += acc[j][e]; }
+      s_acc[(2 * j) * kBlock + tid] += q;
+      s_acc[(2 * j + 1) * kBlock + tid] += sm;
+    }
+  }
+  if (blockIdx.x == 0 && tid == 0)
+    for (uint64_t r = ng * E; r < n; r++)
+      for (int j = 0; j < M; j++) {
+        double a = 0.0;
+        for (uint32_t t = 0; t < k; t++) a += s_w[t * M + j] * (double)V[(uint64_t)t * ldv + r];
+        Y[(uint64_t)j * ldv + r] = a;
+        s_acc[(2 * j) * kBlock] += a * a;
+        s_acc[(2 * j + 1) * kBlock] += a;
+      }
+  __syncthreads();
+  const int lane = tid & 31, wid = tid >> 5;
+  for (int v = wid; v < 2 * M; v += kWarps) {        // CTA partials: one warp per value, fixed order
+    double a = 0.0;
+    for (int i = lane; i < kBlock; i += 32) a += s_acc[v * kBlock + i];
+    a = warp_sum(a);
+    if (lane == 0) partials[(uint64_t)v * gridDim.x + blockIdx.x] = a;
+  }
+  // last CTA: one warp per value, lanes stride the CTA partials in index order (as k_multidot)
+  __syncthreads();
+  if (tid == 0) {
+    __threadfence();
+    const unsigned int tk = atomicAdd(ticket, 1u);
+    s_last = (tk == gridDim.x - 1);
+  }
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  for (int v = wid; v < 2 * M; v += kWarps) {
+    double a = 0.0;
+    for (unsigned int i = lane; i < gridDim.x; i += 32) a += __ldcg(partials + (uint64_t)v * gridDim.x + i);
+    a = warp_sum(a);
+    if (lane == 0) ((v & 1) ? vsum : nrm2)[v >> 1] = a;
+  }
+  if (tid == 0) *ticket = 0u;
+}
+
+// sum_i v[i] (m = 1: the sign of the vector k_combine built)
+__global__ void __launch_bounds__(kBlock) k_vsum(const double* __restrict__ v, uint64_t n, double* partials, unsigned int* ticket, double* out) {
+  __shared__ double sm[kWarps];
+  __shared__ bool s_last;
+  double acc = 0.0;
+  for (uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x; i < n; i += (uint64_t)gridDim.x * kBlock) acc += v[i];
+  acc = block_sum(acc, sm);
+  grid_sum_finish(acc, partials, ticket, out, sm, &s_last);
+}
+
+// max of non-negative doubles through their bit patterns (ordered like the values): exact, so the order of arrival does not matter
+__device__ __forceinline__ void block_max_to(double v, double* sm, unsigned long long* out) {
+  for (int o = 16; o > 0; o >>= 1) v = fmax(v, __shfl_xor_sync(0xffffffffu, v, o));
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  __syncthreads();
+  if (lane == 0) sm[wid] = v;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int w = 1; w < kWarps; w++) v = fmax(v, sm[w]);
+    atomicMax(out, (unsigned long long)__double_as_longlong(v));
+  }
+}
+
+// y_j *= sgn(vsum_j) / sqrt(nrm2_j) for j < m (unit 2-norm, sum_i y_j(i) >= 0); max |y_0| -> *absmax0 (bits of a double)
+__global__ void __launch_bounds__(kBlock) k_ritz_scale(double* __restrict__ Y, uint64_t ldv, uint32_t m, uint64_t n, const double* __restrict__ nrm2,
+                                                       const double* __restrict__ vsum, unsigned long long* absmax0) {
+  __shared__ double sm[kWarps];
+  double mx = 0.0;
+  for (uint32_t j = 0; j < m; j++) {
+    const double s = (vsum[j] < 0.0 ? -1.0 : 1.0) / sqrt(nrm2[j]);
+    double* y = Y + (uint64_t)j * ldv;
+    for (uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x; i < n; i += (uint64_t)gridDim.x * kBlock) {
+      const double v = y[i] * s;
+      y[i] = v;
+      if (j == 0) mx = fmax(mx, fabs(v));
+    }
+  }
+  block_max_to(mx, sm, absmax0);
+}
+
+// Collatz-Wielandt weights z = max(|y_0|, delta * max|y_0|) > 0, entry-wise; z may be y (several GPUs: in place on the gathered vector)
+__global__ void __launch_bounds__(kBlock) k_cw_z(const double* y, double* z, uint64_t n, const double* __restrict__ absmax,
+                                                 double delta) {
+  const double floor_v = delta * *absmax;
+  for (uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x; i < n; i += (uint64_t)gridDim.x * kBlock) z[i] = fmax(fabs(y[i]), floor_v);
+}
+
+// max over this rank's vertices (padding slots excluded) of (A z)_i / z_i -> *out (bits of a double). zfull is the gathered z.
+__global__ void __launch_bounds__(kBlock) k_cw_bound(const double* __restrict__ az, const double* __restrict__ zfull, uint64_t n, uint64_t cl,
+                                                     uint32_t world, uint32_t rank, const uint32_t* __restrict__ new2old,
+                                                     unsigned long long* out) {
+  __shared__ double sm[kWarps];
+  double mx = 0.0;
+  for (uint64_t l = (uint64_t)blockIdx.x * kBlock + threadIdx.x; l < n; l += (uint64_t)gridDim.x * kBlock) {
+    const uint64_t slot = xfull_index(l, cl, world, rank);
+    if (new2old[slot] != 0xFFFFFFFFu) mx = fmax(mx, az[l] / zfull[slot]);
+  }
+  block_max_to(mx, sm, out);
+}
+
 inline unsigned stream_grid(const lz_ctx* c, uint64_t work_items /* per-thread items */) {
   uint64_t want = (work_items + kBlock - 1) / kBlock;
   uint64_t cap = (uint64_t)c->sm_count * 8;
@@ -1682,3 +1856,63 @@ int lz_k_fill(lz_ctx* c, double* p, uint64_t n, double value) {
 }
 
 int lz_k_reserve_partials(lz_ctx* c, uint64_t count) { return ensure_partials(c, count); }
+
+int lz_k_ritz_select(lz_ctx* c, uint32_t k, uint32_t m, uint32_t M, const double* eigvals, const double* eigvecs, const double* norm2, double* W,
+                     double* theta) {
+  k_ritz_select<<<1, kBlock, 0, c->stream>>>(k, m, M, eigvals, eigvecs, norm2, W, theta);
+  LZ_LAUNCH_CHECK();
+  return LZ_OK;
+}
+
+template <class TV, int M>
+static int launch_ritz_combine(lz_ctx* c, const TV* V, uint32_t k, const double* W, double* Y, double* partials, double* nrm2, double* vsum) {
+  const unsigned g = stream_grid(c, c->n_loc / 2 + 1);
+  const size_t smem = ((size_t)k * M + 2 * M * kBlock) * sizeof(double);
+  if (smem > 48 * 1024) LZ_CUDA(cudaFuncSetAttribute(k_ritz_combine<TV, M>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  k_ritz_combine<TV, M><<<g, kBlock, smem, c->stream>>>(V, c->ldv, k, W, Y, c->n_loc, partials, c->ticket + 5, nrm2, vsum);
+  LZ_LAUNCH_CHECK();
+  return LZ_OK;
+}
+
+int lz_k_ritz_combine(lz_ctx* c, const void* V, bool f32, uint32_t k, uint32_t M, const double* W, double* Y, double* partials, double* nrm2,
+                      double* vsum) {
+  if (k > (uint32_t)kEigMax) return lz_fail(LZ_ERR_ARG, "krylov dimension %u exceeds %d", k, kEigMax);
+  static_assert(((size_t)kEigMax * 16 + 2 * 16 * kBlock) * sizeof(double) <= 227 * 1024, "W of the largest k must fit in shared memory");
+#define LZ_RITZ_CASE(MM)                                                                                                  \
+  case MM:                                                                                                                \
+    return f32 ? launch_ritz_combine<float, MM>(c, (const float*)V, k, W, Y, partials, nrm2, vsum)                      \
+               : launch_ritz_combine<double, MM>(c, (const double*)V, k, W, Y, partials, nrm2, vsum);
+  switch (M) {
+    LZ_RITZ_CASE(2)
+    LZ_RITZ_CASE(4)
+    LZ_RITZ_CASE(8)
+    LZ_RITZ_CASE(16)
+    default: return lz_fail(LZ_ERR_ARG, "Ritz block width %u is not 2, 4, 8 or 16", M);
+  }
+#undef LZ_RITZ_CASE
+}
+
+int lz_k_vsum(lz_ctx* c, const double* v, uint64_t n, double* partials, double* out) {
+  k_vsum<<<stream_grid(c, n), kBlock, 0, c->stream>>>(v, n, partials, c->ticket + 5, out);
+  LZ_LAUNCH_CHECK();
+  return LZ_OK;
+}
+
+int lz_k_ritz_scale(lz_ctx* c, double* Y, uint32_t m, const double* nrm2, const double* vsum, unsigned long long* absmax0) {
+  k_ritz_scale<<<stream_grid(c, c->n_loc), kBlock, 0, c->stream>>>(Y, c->ldv, m, c->n_loc, nrm2, vsum, absmax0);
+  LZ_LAUNCH_CHECK();
+  return LZ_OK;
+}
+
+int lz_k_cw_z(lz_ctx* c, const double* y, double* z, uint64_t n, const double* absmax, double delta) {
+  k_cw_z<<<stream_grid(c, n), kBlock, 0, c->stream>>>(y, z, n, absmax, delta);
+  LZ_LAUNCH_CHECK();
+  return LZ_OK;
+}
+
+int lz_k_cw_bound(lz_ctx* c, const double* az, const double* zfull, unsigned long long* out) {
+  k_cw_bound<<<stream_grid(c, c->n_loc), kBlock, 0, c->stream>>>(az, zfull, c->n_loc, c->chunk_rows, (uint32_t)c->world, (uint32_t)c->rank,
+                                                                c->new2old, out);
+  LZ_LAUNCH_CHECK();
+  return LZ_OK;
+}

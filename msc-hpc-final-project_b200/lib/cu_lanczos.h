@@ -27,6 +27,7 @@ T norm(const T* v, U n) {  // cu_lanczos.h:18-24
 
 template <typename U, typename V> void check_ans(lanczosDecomp<U>&, lanczosDecomp<V>&);
 template <typename U> void write_ans(std::string filename, lanczosDecomp<U>&);
+template <typename T> class ritzPairs;
 
 template <typename T>
 class lanczosDecomp {
@@ -92,6 +93,7 @@ class lanczosDecomp {
   lz_timings timings() const { lz_timings t{}; lz_timings_get(ctx, &t); return t; }
 
   friend class eigenDecomp<T>;
+  friend class ritzPairs<T>;
   template <typename U> friend void multOut(lanczosDecomp<U>&, eigenDecomp<U>&, adjMatrix&, bool);
   template <typename U, typename V> friend void check_ans(lanczosDecomp<U>&, lanczosDecomp<V>&);
   template <typename U> friend void write_ans(std::string filename, lanczosDecomp<U>&);

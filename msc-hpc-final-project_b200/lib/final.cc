@@ -10,6 +10,9 @@
 //            --write FILE (one value per line, write_ans)   --top M (print the M most central vertices, device-side ranking)
 //            --t T (e^{TA} x, inverse temperature T)   --scaled (e^{T(A - sI)} x, s = largest Ritz value: never overflows; the log
 //            scale T*s is printed)   --katz ALPHA ((I - ALPHA A)^{-1} x, Katz centrality)
+//            --ritz M (the top M Ritz pairs with their certified eigenvalue intervals)   --eigcent (eigenvector centrality: the result
+//            and --top are y_0; prints the spectral-radius bracket)   --katz-frac F (Katz with alpha = F / hi, hi the certified upper
+//            bound on lambda_max, so F < 1 guarantees alpha < 1 / lambda_max; prints alpha and the bracket)
 //
 // Same object sequence as the reference: adjMatrix -> lanczosDecomp<double>(A,k,x,cuda=true) -> eigenDecomp<double> ->
 // multOut(L,E,A,true), same TIMING / ERROR CHECKING tables. The reference's serial arm (main.cu:83-99) is not here: this
@@ -30,15 +33,33 @@
 #include "eigen.h"
 #include "helpers.h"
 #include "multiplyOut.h"
+#include "ritz.h"
 #include "write_ans.h"
 
 #define WIDTH 81
 
 static double seconds_between(timeval s, timeval e) { return e.tv_sec - s.tv_sec + (e.tv_usec - s.tv_usec) / 1000000.0; }
 
-// Row-sharded run over `gpus` devices: one host thread per GPU, each driving its own lz_ctx (C ABI directly).
+struct ritz_out {
+  std::vector<double> theta, rho, res;
+  double lo = 0.0, hi = 0.0;
+};
+
+static void print_ritz(const ritz_out& R, bool pairs) {
+  std::cout << std::setprecision(17);
+  if (pairs) {
+    std::cout << "Ritz pairs (j theta rayleigh residual; [rayleigh - residual, rayleigh + residual] holds an eigenvalue of A)\n";
+    for (size_t j = 0; j < R.theta.size(); j++)
+      std::cout << "ritz " << j << ' ' << R.theta[j] << ' ' << R.rho[j] << ' ' << R.res[j] << " [" << R.rho[j] - R.res[j] << ", "
+                << R.rho[j] + R.res[j] << "]\n";
+  }
+  std::cout << "spectral radius bracket: " << R.lo << ' ' << R.hi << '\n' << std::setprecision(6);
+}
+
+// Row-sharded run over `gpus` devices: one host thread per GPU, each driving its own lz_ctx (C ABI directly). ritz_m > 0: lz_ritz
+// after the run; katz_frac > 0: then Katz with alpha = katz_frac / hi; eigcent: the result is y_0 (no coefficient solve).
 static int run_multi(adjMatrix& A, unsigned k, int reorth, int gpus, int fkind, double fparam, std::vector<double>& ans, double& log_scale,
-                     double& t_lanczos, double& t_mult) {
+                     double& t_lanczos, double& t_mult, unsigned ritz_m, double katz_frac, bool eigcent, ritz_out& R) {
   unsigned char uid[LZ_NCCL_UID_BYTES];
   if (lz_nccl_unique_id(uid) != LZ_OK) { std::cerr << lz_last_error() << '\n'; return 1; }
   std::vector<int> rc(gpus, 0);
@@ -60,14 +81,25 @@ static int run_multi(adjMatrix& A, unsigned k, int reorth, int gpus, int fkind, 
       if ((e = lz_lanczos_run(c, k, reorth)) != LZ_OK) return bad(e);
       if ((e = lz_sync(c)) != LZ_OK) return bad(e);
       gettimeofday(&e1, NULL);
-      if ((e = lz_tridiag_expv(c)) != LZ_OK) return bad(e);
-      if ((e = lz_multout(c)) != LZ_OK) return bad(e);
+      if (ritz_m) {
+        ritz_out mine;
+        mine.theta.resize(ritz_m); mine.rho.resize(ritz_m); mine.res.resize(ritz_m);
+        if ((e = lz_ritz(c, ritz_m)) != LZ_OK) return bad(e);
+        if ((e = lz_get_ritz(c, mine.theta.data(), mine.rho.data(), mine.res.data())) != LZ_OK) return bad(e);
+        if ((e = lz_spectral_radius_bounds(c, &mine.lo, &mine.hi)) != LZ_OK) return bad(e);
+        if (katz_frac > 0.0 && (e = lz_set_matfun(c, LZ_MATFUN_RESOLVENT, katz_frac / mine.hi)) != LZ_OK) return bad(e);
+        if (r == 0) R = mine;
+      }
+      if (!eigcent) {
+        if ((e = lz_tridiag_expv(c)) != LZ_OK) return bad(e);
+        if ((e = lz_multout(c)) != LZ_OK) return bad(e);
+      }
       std::vector<double> y(A.get_n());
       if ((e = lz_get_ans(c, y.data())) != LZ_OK) return bad(e);
       gettimeofday(&e2, NULL);
       tl[r] = seconds_between(s, e1); tm[r] = seconds_between(e1, e2);
       if (r == 0) {
-        if ((e = lz_get_matfun_scale(c, &log_scale)) != LZ_OK) return bad(e);
+        if (!eigcent && (e = lz_get_matfun_scale(c, &log_scale)) != LZ_OK) return bad(e);
         ans.swap(y);
       }
       lz_destroy(c);
@@ -89,8 +121,9 @@ int main(int argc, char** argv) {
   uint64_t seed = 1;
   int reorth = LZ_REORTH_NONE, gpus = 1;
   unsigned top = 0;
-  double t = 1.0, katz = 0.0;
-  bool scaled = false, have_t = false, have_katz = false;
+  double t = 1.0, katz = 0.0, katz_frac = 0.0;
+  bool scaled = false, have_t = false, have_katz = false, have_katz_frac = false, eigcent = false;
+  unsigned ritz_req = 0;
 
   // long options first; what is left goes to the reference's getopt string
   std::vector<char*> rest{argv[0]};
@@ -117,16 +150,20 @@ int main(int argc, char** argv) {
     else if (a == "--t") { t = num(); have_t = true; }
     else if (a == "--scaled") scaled = true;
     else if (a == "--katz") { katz = num(); have_katz = true; }
+    else if (a == "--katz-frac") { katz_frac = num(); have_katz_frac = true; }
+    else if (a == "--eigcent") eigcent = true;
+    else if (a == "--ritz") { const double v = num(); ritz_req = (unsigned)v; if (v < 1 || v > LZ_RITZ_MAX || v != ritz_req) { std::cerr << "--ritz takes 1.." << LZ_RITZ_MAX << '\n'; return 2; } }
     else rest.push_back(argv[i]);
   }
   if (parseArguments((int)rest.size(), rest.data(), filename, krylov_dim, verbose, n, deg, edges) != 0) return 2;
   if (have_katz && (have_t || scaled)) { std::cerr << "--katz excludes --t and --scaled\n"; return 2; }
-  const int fkind = have_katz ? LZ_MATFUN_RESOLVENT : scaled ? LZ_MATFUN_EXP_SCALED : LZ_MATFUN_EXP;
-  const double fparam = have_katz ? katz : t;
-  const bool default_fun = fkind == LZ_MATFUN_EXP && fparam == 1.0;
-  std::string fun_label = "total communicability";
-  if (have_katz) fun_label = "Katz centrality (I - alpha A)^-1 x, alpha = " + std::to_string(fparam);
-  else if (!default_fun) fun_label = "total communicability e^{tA} x, t = " + std::to_string(fparam) + (scaled ? ", scaled by e^-log_scale" : "");
+  if (have_katz_frac && (have_katz || have_t || scaled)) { std::cerr << "--katz-frac excludes --katz, --t and --scaled\n"; return 2; }
+  if (have_katz_frac && !(katz_frac > 0.0 && katz_frac < 1.0)) { std::cerr << "--katz-frac takes a fraction in (0, 1)\n"; return 2; }
+  if (eigcent && (have_katz || have_katz_frac || have_t || scaled)) { std::cerr << "--eigcent excludes --katz, --katz-frac, --t and --scaled\n"; return 2; }
+  const unsigned ritz_m = ritz_req ? ritz_req : (eigcent || have_katz_frac) ? 1u : 0u;
+  const int fkind = (have_katz || have_katz_frac) ? LZ_MATFUN_RESOLVENT : scaled ? LZ_MATFUN_EXP_SCALED : LZ_MATFUN_EXP;
+  double fparam = have_katz ? katz : t;
+  const bool default_fun = fkind == LZ_MATFUN_EXP && fparam == 1.0 && !eigcent;
 
   timeval start, end;
   gettimeofday(&start, NULL);
@@ -167,25 +204,51 @@ int main(int argc, char** argv) {
   std::vector<double> result;
   double gpu_time_lanczos = 0, gpu_time_mult = 0, gpu_time_whole = 0, log_scale = 0;
   lz_timings tm{};
+  ritz_out rz;
+  auto label = [&]() {
+    if (eigcent) return std::string("eigenvector centrality");
+    if (fkind == LZ_MATFUN_RESOLVENT) return "Katz centrality (I - alpha A)^-1 x, alpha = " + std::to_string(fparam);
+    if (!default_fun) return "total communicability e^{tA} x, t = " + std::to_string(fparam) + (scaled ? ", scaled by e^-log_scale" : "");
+    return std::string("total communicability");
+  };
+  std::string fun_label;
   if (gpus > 1) {
-    if (run_multi(A, krylov_dim, reorth, gpus, fkind, fparam, result, log_scale, gpu_time_lanczos, gpu_time_mult)) return 1;
+    if (run_multi(A, krylov_dim, reorth, gpus, fkind, fparam, result, log_scale, gpu_time_lanczos, gpu_time_mult, ritz_m, katz_frac, eigcent, rz))
+      return 1;
+    if (have_katz_frac) fparam = katz_frac / rz.hi;
+    fun_label = label();
     gpu_time_whole = gpu_time_lanczos + gpu_time_mult;
   } else {
     timeval s, e1, e2, e3;
     gettimeofday(&s, NULL);
     lanczosDecomp<double> cu_L(A, krylov_dim, &x_double[0], /*cuda=*/true, reorth);   // main.cu:115
     gettimeofday(&e1, NULL);
-    eigenDecomp<double> cu_E(cu_L, fkind, fparam);                                    // main.cu:124
-    gettimeofday(&e2, NULL);
-    multOut(cu_L, cu_E, A, true);                                                     // main.cu:127
-    gettimeofday(&e3, NULL);
+    if (ritz_m) {
+      ritzPairs<double> R(cu_L, ritz_m);
+      rz.theta = R.values(); rz.rho = R.rayleigh(); rz.res = R.residuals();
+      R.spectral_radius_bounds(rz.lo, rz.hi);
+      if (have_katz_frac) fparam = katz_frac / rz.hi;                                 // certified: alpha < 1 / lambda_max
+      if (eigcent) {
+        result.resize(n);
+        R.vector(0, result.data());
+      }
+    }
+    fun_label = label();
+    if (eigcent) {                                                                    // the answer (and top_k) is y_0 until a multOut
+      e2 = e3 = e1;
+    } else {
+      eigenDecomp<double> cu_E(cu_L, fkind, fparam);                                  // main.cu:124
+      gettimeofday(&e2, NULL);
+      multOut(cu_L, cu_E, A, true);                                                   // main.cu:127
+      gettimeofday(&e3, NULL);
+      result.assign(cu_L.get_ans_ptr(), cu_L.get_ans_ptr() + n);
+      log_scale = cu_E.log_scale();
+    }
     gpu_time_lanczos = seconds_between(s, e1);
     gpu_time_mult = seconds_between(e2, e3);
     gpu_time_whole = seconds_between(s, e3);
     tm = cu_L.timings();
-    result.assign(cu_L.get_ans_ptr(), cu_L.get_ans_ptr() + n);
-    log_scale = cu_E.log_scale();
-    if (!write_file.empty()) write_ans(write_file, cu_L);                             // main.cu:159
+    if (!write_file.empty() && !eigcent) write_ans(write_file, cu_L);                             // main.cu:159
     if (top) {
       std::vector<unsigned> ti(top);
       std::vector<double> tv(top);
@@ -196,7 +259,10 @@ int main(int argc, char** argv) {
     }
   }
 
-  if (!default_fun)
+  if (ritz_m) print_ritz(rz, ritz_req > 0);
+  if (have_katz_frac) std::cout << "katz alpha: " << std::setprecision(17) << fparam << std::setprecision(6) << " (= " << katz_frac << " / hi)\n";
+  if (eigcent) std::cout << "result: eigenvector centrality y_0 (unit 2-norm)\n";
+  else if (!default_fun)
     std::cout << "matrix function: " << fun_label << "\nlog scale: " << std::setprecision(17) << log_scale << std::setprecision(6)
               << " (f(A) x = result * e^log_scale)\n";
   std::cout << std::setfill('~') << std::setw(WIDTH) << '\n' << std::setfill(' ');
@@ -229,7 +295,7 @@ int main(int argc, char** argv) {
               << std::setw(30) << r.relative_norm << std::endl;
     if (!(r.relative_norm < 1e-9)) status = 4;
   }
-  if (gpus > 1 && !write_file.empty()) {
+  if ((gpus > 1 || eigcent) && !write_file.empty()) {
     std::ofstream fs(write_file);
     fs << std::setprecision(17);
     for (double v : result) fs << v << '\n';
