@@ -128,7 +128,10 @@ int lz_csr_download(lz_ctx* ctx, uint32_t* row_offset_out, uint32_t* col_idx_out
 #define LZ_BASIS_F64 0
 #define LZ_BASIS_F32 1
 int lz_set_basis_precision(lz_ctx* ctx, int precision);
-/* x (n doubles, original order; NULL = all ones as in main.cu:79) -> device, computes ||x|| (cu_lanczos.h:18-24,63). */
+/* x (n doubles, original order; NULL = all ones as in main.cu:79) -> device, computes ||x|| (cu_lanczos.h:18-24,63). ||x|| is taken
+ * as 2^e ||2^-e x|| with e the exponent of max|x_i|, so it neither underflows nor overflows for any finite x: f(A)(2^p x) is
+ * 2^p f(A) x to the bit while the values stay normal, and for every x whose squares are normal the bits are those of the plain sum
+ * of squares. A host vector costs one read-back of max|x_i| (synchronises). LZ_ERR_ARG for a zero or non-finite x. */
 int lz_set_start_vector(lz_ctx* ctx, const double* x_host);
 /* Multi-GPU: only rank `root` reads x_host (one PCIe upload); the other ranks receive the vector over NVLink. Collective. */
 int lz_set_start_vector_root(lz_ctx* ctx, const double* x_host, int root);
@@ -189,13 +192,16 @@ int lz_top_k(lz_ctx* ctx, uint32_t m, uint32_t* idx_out, double* val_out, uint32
 /* ---- top Ritz pairs: eigenvector centrality and a certified spectral-radius bracket ----------------------------------------------
  * After lz_lanczos_run(k) let T = Z Theta Z^T (Theta ascending). For j = 0..m-1: theta_j is the j-th largest Ritz value and
  * y_j = V z_j / ||V z_j|| its Ritz vector, unit 2-norm, sign chosen so that sum_i y_j(i) >= 0. Then, with a real SpMV,
- *   rho_j = y_j^T A y_j             the Rayleigh quotient,
+ *   rho_j = y_j^T A y_j             the Rayleigh quotient (computed),
  *   r_j   = ||A y_j - rho_j y_j||_2 the true residual (not the Lanczos estimate beta_k |e_k^T z_j|, which needs the beta_k the run does not
- *                                   compute and is not valid once orthogonality is lost).
+ *                                   compute and is not valid once orthogonality is lost), computed and then enlarged by the fp64
+ *                                   rounding allowance r_j (2n + 24) 2^-52 + (max_degree + 8) 2^-52 hi. It covers the SpMV's row
+ *                                   sums, the dot product, the residual's sum of squares and ||y_j|| != 1 in fp64 (DESIGN.md).
  * A is symmetric, so [rho_j - r_j, rho_j + r_j] contains an eigenvalue of A (Krylov-Bogoliubov) for plain and reorthogonalised runs,
- * fp64 or fp32 basis, lagged or not. A plain run can return two copies of a converged eigenvalue when m > 1 ("ghosts"); each interval
+ * fp64 or fp32 basis, lagged or not; so does that interval with its ends rounded to fp64. A plain run can return two copies of a converged eigenvalue when m > 1 ("ghosts"); each interval
  * is still correct. Use LZ_REORTH_FULL and a random start vector when the pairs beyond the first matter.
- * Spectral-radius bracket lo <= lambda_max <= hi, for every graph (connected or not): lo = rho_0; hi = max_i (A z)_i / z_i over the
+ * Spectral-radius bracket lo <= lambda_max <= hi, for every graph (connected or not): lo = rho_0 (1 - (2n + max_degree + 24) 2^-52)
+ * (lo = rho_0 when rho_0 <= 0), which covers the rounding of rho_0 as above; hi = max_i (A z)_i / z_i over the
  * vertices (Collatz-Wielandt, A >= 0, z > 0) with z_i = max(|y_0(i)|, LZ_CW_FLOOR * max|y_0|), inflated by the fp64 rounding
  * allowance (max_degree + 2) * 2^-52 (relative). Tight when y_0 has converged on a connected graph. hi certifies a Katz parameter:
  * alpha = f / hi with f < 1 gives alpha < 1 / lambda_max.

@@ -482,7 +482,9 @@ extern "C" int lz_set_spmv_variant(lz_ctx* c, int variant) {
   return LZ_OK;
 }
 
-// x -> device, ||x||^2 -> scal[2], q_0 = x/||x|| -> V[0] (and the gathered buffer when world > 1).
+// x -> device, ||2^-e x||^2 -> scal[2] with e = x_exp the exponent of max|x|, q_0 = x/||x|| -> V[0] (and the gathered buffer when
+// world > 1). Squaring x as it is underflows below |x_i| ~ 1e-154 (||x|| loses digits, q_0 is not a unit vector) and overflows above
+// ~1e154; 2^-e x has max in [1, 2) and the same q_0. For every x whose squares stay normal the bits are those of the unscaled sum.
 // Replaces cu_lanczos.cu:30-34 (host normalisation) + :88 (H2D of q_0).
 // root < 0: every rank passes the vector itself (or NULL = ones). root >= 0: only `root` reads x_host; the other ranks
 // receive it over NVLink (one PCIe upload instead of `world` concurrent ones).
@@ -502,7 +504,19 @@ static int set_start_vector_impl(lz_ctx* c, const double* x_host, int root) {
   } else {
     LZ_TRY(lz_k_fill(c, c->xstage, c->n, 1.0));   // all ones, as every reference driver uses (main.cu:79)
   }
-  LZ_TRY(lz_k_norm2(c, c->xstage, c->n, c->scal + 2));
+  c->x_exp = 0;
+  c->have_x = c->have_tridiag = c->have_coef = c->have_ans = false;
+  if (x_host || (root >= 0 && c->world > 1)) {    // a caller's vector: one read-back of max|x| (ones: e = 0)
+    auto* mx_d = reinterpret_cast<unsigned long long*>(c->scal + 6);
+    LZ_CUDA(cudaMemsetAsync(mx_d, 0, 8, c->stream));
+    LZ_TRY(lz_k_absmax_bits(c, c->xstage, c->n, mx_d));
+    double mx = 0.0;
+    LZ_CUDA(cudaMemcpyAsync(&mx, mx_d, 8, cudaMemcpyDeviceToHost, c->stream));
+    LZ_CUDA(cudaStreamSynchronize(c->stream));
+    if (!(mx > 0.0) || !isfinite(mx)) return lz_fail(LZ_ERR_ARG, "start vector is zero or not finite (max |x_i| = %g)", mx);
+    c->x_exp = ilogb(mx);
+  }
+  LZ_TRY(lz_k_norm2(c, c->xstage, c->n, c->x_exp, c->scal + 2));
   double* q0 = c->basis_f32 ? c->q0_64 : c->V;
   if (c->world > 1) {
     LZ_TRY(lz_k_permute_in_local(c, c->xstage, c->scal + 2, q0));   // own rows only; the gathered vector is filled by the run
@@ -996,16 +1010,31 @@ extern "C" int lz_ritz(lz_ctx* c, uint32_t m) {
     if (!(h[j] > 0.0) || !isfinite(h[j])) return lz_fail(LZ_ERR_NUMERIC, "Ritz vector %u is zero or not finite (||V z||^2 = %g)", j, h[j]);
     if (!isfinite(h[32 + j]) || !isfinite(h[48 + j]) || !isfinite(h[64 + j]))
       return lz_fail(LZ_ERR_NUMERIC, "Ritz pair %u is not finite (theta %g, rho %g, r^2 %g)", j, h[32 + j], h[48 + j], h[64 + j]);
-    c->ritz_theta[j] = h[32 + j];
-    c->ritz_rho[j] = h[48 + j];
-    c->ritz_res[j] = sqrt(h[64 + j]);
   }
   // (A z)_i is a sum of deg_i exact products: computed ratio >= true ratio * (1 - (deg_i + 1) 2^-53); the allowance covers it and the
   // rounding of the product below
   const double cw = h[81];
   if (!isfinite(cw)) return lz_fail(LZ_ERR_NUMERIC, "Collatz-Wielandt bound is not finite");
-  c->ritz_lo = c->ritz_rho[0];
-  c->ritz_hi = cw * (1.0 + ((double)c->max_degree + 2.0) * 0x1p-52);
+  const double ulp = 0x1p-52, D = (double)c->max_degree, N = (double)c->n;
+  const double hi = cw * (1.0 + (D + 2.0) * ulp);
+  // Rounding allowance of the intervals and of lo (u = 2^-53, y the stored Ritz vector, w^ the computed A y, lambda_max <= hi = ||A||_2):
+  //  - the SpMV: |w^ - A y| <= gamma_D A|y| entry-wise, so ||w^ - A y|| <= gamma_D hi ||y||;
+  //  - the residual combine and its sum of squares: ||w^ - rho y|| <= r^ (1 + gamma_n + 3u) + 2u |rho| ||y||;
+  //  - the dot product: |rho - y^T A y| <= c lambda_max ||y||^2 with c = gamma_n (1 + gamma_D) + gamma_D (|y|^T A |y| <= lambda_max ||y||^2);
+  //  - the norm: | ||y||^2 - 1 | <= gamma_n + 8u after k_ritz_scale.
+  // Krylov-Bogoliubov holds for any centre: some eigenvalue lies within ||A y - rho y|| / ||y|| of rho, which the radius below bounds
+  // (with 2u |rho| more, so that rho -/+ r rounded to fp64 still encloses it). For lo, the error of rho is relative to lambda_max, not
+  // to rho: y^T A y <= lambda_max ||y||^2 gives rho <= lambda_max ||y||^2 (1 + c) <= lambda_max (1 + gamma_n + 8u)(1 + c), so
+  // lambda_max >= rho / ((1 + gamma_n + 8u)(1 + c)) >= rho (1 - (2n + D + 24) 2^-52) when rho > 0; a non-negative A has
+  // lambda_max >= 0 >= rho otherwise. The extra units absorb the rounding of these formulas.
+  for (uint32_t j = 0; j < m; j++) {
+    c->ritz_theta[j] = h[32 + j];
+    c->ritz_rho[j] = h[48 + j];
+    c->ritz_res[j] = sqrt(h[64 + j]) * (1.0 + (2.0 * N + 24.0) * ulp) + (D + 8.0) * ulp * hi;
+  }
+  const double rho0 = c->ritz_rho[0];
+  c->ritz_lo = rho0 > 0.0 ? rho0 * (1.0 - (2.0 * N + D + 24.0) * ulp) : rho0;
+  c->ritz_hi = hi;
   c->ritz_m = m;
   c->ritz_run = c->run_serial;
   c->have_ans = true;

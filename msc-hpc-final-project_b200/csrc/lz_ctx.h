@@ -151,8 +151,9 @@ struct lz_ctx {
   bool lagged = true;              // use the lagged normalisation where it applies (one GPU, no reorthogonalisation); LZ_LAGGED_NORM=0 disables
   bool lagged_done = false;        // the last run left rows 1.. of V unnormalised
   bool lagged_run = false;         // set by the step loop that is being enqueued
-  double* scal = nullptr;          // device scalars: [0]=alpha acc, [1]=norm2 acc, [2]=x_norm, [5]=log scale of the last
-                                   // coefficient solve (lz_get_matfun_scale), others: scratch of the step loop and set-up
+  double* scal = nullptr;          // device scalars: [0]=alpha acc, [1]=norm2 acc, [2]=||2^-x_exp x||^2, [5]=log scale of the last
+                                   // coefficient solve (lz_get_matfun_scale), [6]=max|x| (bits), others: scratch of the step loop and set-up
+  int x_exp = 0;                   // exponent of max|x|: x is scaled by 2^-x_exp before squaring, so ||x|| neither overflows nor underflows
   double* partials = nullptr;      // device, per-CTA partial sums
   uint32_t partials_cap = 0;
   unsigned int* ticket = nullptr;  // device, last-block counters
@@ -233,12 +234,15 @@ int lz_k_scale(lz_ctx* c, const double* w, const double* norm2, double* q_next, 
 int lz_k_scale_push(lz_ctx* c, const double* w, const double* norm2, double* q_next, double* beta_out, unsigned long long seq,
                     uint32_t push_chunks /* chunks [0, push_chunks) are sent here; the rest by the SpMV passes */,
                     unsigned long long red_seq = 0);
-// q0_local[l] = x_orig[new2old[slot(l)]] / sqrt(*norm2)
+// q0_local[l] = 2^-x_exp x_orig[new2old[slot(l)]] / sqrt(*norm2)
 int lz_k_permute_in_local(lz_ctx* c, const double* x_orig, const double* norm2, double* q0_local);
 // local vector <-> this rank's slots of the chunk-major gathered vector
 int lz_k_spread(lz_ctx* c, const double* local, double* xfull);
 int lz_k_collect(lz_ctx* c, const double* xfull, double* local);
-int lz_k_norm2(lz_ctx* c, const double* v, uint64_t len, double* out);
+// *out = ||2^-e v||^2
+int lz_k_norm2(lz_ctx* c, const double* v, uint64_t len, int e, double* out);
+// *out = max(*out, bits of max_i |v[i]|) (NaN > inf > finite as integers)
+int lz_k_absmax_bits(lz_ctx* c, const double* v, uint64_t len, unsigned long long* out);
 // V: the basis, [nvec][ldv] doubles, or floats when f32 (LZ_BASIS_F32)
 int lz_k_multidot(lz_ctx* c, const void* V, bool f32, uint32_t nvec, const double* w, double* h_out /* device [nvec] */, const int* skip = nullptr,
                   const double* h_div = nullptr /* h[t] /= h_div[t]: unnormalised basis rows */);
@@ -253,7 +257,7 @@ int lz_k_tridiag_expv(lz_ctx* c, uint32_t k);   // the ctx's result; log scale -
 // ls_in: shift to use for LZ_MATFUN_EXP_SCALED instead of the block's own (null: own); ls_out (may be null) receives the one used
 int lz_k_tridiag_expv_into(lz_ctx* c, uint32_t k, double* eigvals, double* eigvecs, double* work, double* coef, int* status,
                            const double* ls_in, double* ls_out);
-// dst[i] = x_orig[new2old[first + i]] (/ sqrt(*norm2) when norm2 != null), i < count; padding slots -> 0
+// dst[i] = x_orig[new2old[first + i]] (times 2^-x_exp / sqrt(*norm2) when norm2 != null), i < count; padding slots -> 0
 int lz_k_permute_in(lz_ctx* c, const double* x_orig, const double* norm2, uint64_t first, uint64_t count, double* dst);
 int lz_k_permute_out(lz_ctx* c, const double* y_new_full, double* y_orig);
 int lz_k_fill(lz_ctx* c, double* p, uint64_t n, double value);

@@ -534,7 +534,9 @@ static int finish_local(lz_ctx* c, const Order& o, DevBuf& k_in, uint64_t nkeys,
         c->sell_narrow[b] = force >= 0 ? force != 0 : (natural && slices > 0 && (double)(hi - lo) / slices <= 6.0);
       }
     }
-    if (c->sell_entries > 6 * c->nnz_loc + 64 * (uint64_t)tot_items + 1024)   // 32-bit chunk counter wrapped, or absurd padding
+    // 32-bit chunk counter wrapped, or absurd padding. The first slice of a block may be as wide as a row of LZ_SELL_LONG entries (a star
+    // K_{1,100}: 3296 entries for 200 non-zeros), so that much padding per block is always allowed.
+    if (c->sell_entries > 6 * c->nnz_loc + 64 * (uint64_t)tot_items + 1024 + 32ull * LZ_SELL_LONG * nblk)
       return lz_fail(LZ_ERR_ARG, "sliced layout too large (%llu entries for %llu non-zeros)", (unsigned long long)c->sell_entries,
                      (unsigned long long)c->nnz_loc);
     LZ_CUDA(cudaMalloc((void**)&c->sell_col, (c->sell_entries ? c->sell_entries : 1) * 4));

@@ -998,13 +998,13 @@ __global__ void __launch_bounds__(kBlock) k_scale_push_sparse(const double* __re
   }
 }
 
-// q0_local[l] = x_orig[new2old[slot(l)]] / sqrt(norm2)
+// q0_local[l] = 2^-xexp x_orig[new2old[slot(l)]] / sqrt(norm2)
 __global__ void k_permute_in_local(const double* __restrict__ x_orig, const uint32_t* __restrict__ new2old, uint64_t n, uint64_t cl,
-                                   uint32_t world, uint32_t rank, const double* __restrict__ norm2_p, double* __restrict__ dst) {
+                                   uint32_t world, uint32_t rank, const double* __restrict__ norm2_p, int xexp, double* __restrict__ dst) {
   const double nrm = sqrt(*norm2_p);
   for (uint64_t l = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; l < n; l += (uint64_t)gridDim.x * blockDim.x) {
     const uint32_t o = new2old[xfull_index(l, cl, world, rank)];
-    dst[l] = (o == 0xFFFFFFFFu) ? 0.0 : x_orig[o] / nrm;
+    dst[l] = (o == 0xFFFFFFFFu) ? 0.0 : ldexp(x_orig[o], -xexp) / nrm;
   }
 }
 
@@ -1019,23 +1019,42 @@ __global__ void __launch_bounds__(kBlock) k_spread_collect(double* __restrict__ 
   }
 }
 
-__global__ void __launch_bounds__(kBlock) k_norm2(const double* __restrict__ v, uint64_t n, double* partials, unsigned int* ticket,
+// ||2^-e v||^2. Scaling by a power of two is exact, so for an e that keeps the squares normal the result is 2^-2e ||v||^2 to the bit.
+__global__ void __launch_bounds__(kBlock) k_norm2(const double* __restrict__ v, uint64_t n, int e, double* partials, unsigned int* ticket,
                                                   double* out) {
   __shared__ double sm[kWarps];
   __shared__ bool s_last;
   double acc = 0.0;
-  for (uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x; i < n; i += (uint64_t)gridDim.x * kBlock) acc += v[i] * v[i];
+  for (uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x; i < n; i += (uint64_t)gridDim.x * kBlock) {
+    const double a = ldexp(v[i], -e);
+    acc += a * a;
+  }
   acc = block_sum(acc, sm);
   grid_sum_finish(acc, partials, ticket, out, sm, &s_last);
 }
 
-// dst[i] = x_orig[new2old[first + i]] / sqrt(norm2) for i < count (0 for padding slots)
+// max_i |v[i]| as the bit pattern of a non-negative double, ordered like the values with NaN above inf: *out must be zeroed first
+__global__ void __launch_bounds__(kBlock) k_absmax_bits(const double* __restrict__ v, uint64_t n, unsigned long long* out) {
+  __shared__ unsigned long long sm[kWarps];
+  unsigned long long mx = 0ull;
+  for (uint64_t i = (uint64_t)blockIdx.x * kBlock + threadIdx.x; i < n; i += (uint64_t)gridDim.x * kBlock)
+    mx = max(mx, (unsigned long long)__double_as_longlong(v[i]) & 0x7FFFFFFFFFFFFFFFull);
+  for (int o = 16; o > 0; o >>= 1) mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, o));
+  if ((threadIdx.x & 31) == 0) sm[threadIdx.x >> 5] = mx;
+  __syncthreads();
+  if (threadIdx.x == 0) {
+    for (int w = 1; w < kWarps; w++) mx = max(mx, sm[w]);
+    atomicMax(out, mx);
+  }
+}
+
+// dst[i] = 2^-xexp x_orig[new2old[first + i]] / sqrt(norm2) for i < count (0 for padding slots)
 __global__ void k_permute_in(const double* __restrict__ x_orig, const uint32_t* __restrict__ new2old, uint64_t first, uint64_t count,
-                             const double* __restrict__ norm2_p, double* __restrict__ dst) {
+                             const double* __restrict__ norm2_p, int xexp, double* __restrict__ dst) {
   const double nrm = sqrt(*norm2_p);
   for (uint64_t i = (uint64_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (uint64_t)gridDim.x * blockDim.x) {
     const uint32_t o = new2old[first + i];
-    dst[i] = (o == 0xFFFFFFFFu) ? 0.0 : x_orig[o] / nrm;
+    dst[i] = (o == 0xFFFFFFFFu) ? 0.0 : ldexp(x_orig[o], -xexp) / nrm;
   }
 }
 // same without scaling
@@ -1217,7 +1236,7 @@ __global__ void __launch_bounds__(kBlock) k_combine(const TV* __restrict__ V, ui
 // ls goes to *ls_out (when given) so that e^{pA} x = ans * e^ls.
 constexpr int kEigMax = 1024;
 __global__ void __launch_bounds__(kBlock) k_tridiag_expv(uint32_t k, const double* __restrict__ alpha, const double* __restrict__ beta,
-                                                         const double* __restrict__ xnorm2_p, double* __restrict__ eigvals,
+                                                         const double* __restrict__ xnorm2_p, int xexp, double* __restrict__ eigvals,
                                                          double* __restrict__ eigvecs, double* __restrict__ zt_global, double* __restrict__ coef,
                                                          int* __restrict__ status, int zt_in_smem, int fkind, double fparam,
                                                          const double* __restrict__ ls_in, double* __restrict__ ls_out) {
@@ -1346,7 +1365,7 @@ __global__ void __launch_bounds__(kBlock) k_tridiag_expv(uint32_t k, const doubl
     if (ls_out) *ls_out = ls;
   }
   __syncthreads();
-  const double xn = sqrt(*xnorm2_p), ls = s_ls;
+  const double xn = ldexp(sqrt(*xnorm2_p), xexp), ls = s_ls;   // ||x|| = 2^xexp ||2^-xexp x||
   bool indefinite = false;
   for (int j = tid; j < n; j += kBlock) {   // f_j ; row 0 of eigvecs
     const double lam = d[perm[j]];
@@ -1752,7 +1771,7 @@ int lz_k_scale_push(lz_ctx* c, const double* w, const double* norm2, double* q_n
 
 int lz_k_permute_in_local(lz_ctx* c, const double* x_orig, const double* norm2, double* q0_local) {
   k_permute_in_local<<<stream_grid(c, c->n_loc), kBlock, 0, c->stream>>>(x_orig, c->new2old, c->n_loc, c->chunk_rows, (uint32_t)c->world,
-                                                                        (uint32_t)c->rank, norm2, q0_local);
+                                                                        (uint32_t)c->rank, norm2, c->x_exp, q0_local);
   LZ_LAUNCH_CHECK();
   return LZ_OK;
 }
@@ -1773,10 +1792,16 @@ int lz_k_collect(lz_ctx* c, const double* xfull, double* local) {
   return LZ_OK;
 }
 
-int lz_k_norm2(lz_ctx* c, const double* v, uint64_t len, double* out) {
+int lz_k_norm2(lz_ctx* c, const double* v, uint64_t len, int e, double* out) {
   unsigned g = stream_grid(c, len);
   LZ_TRY(ensure_partials(c, g));
-  k_norm2<<<g, kBlock, 0, c->stream>>>(v, len, c->partials, c->ticket + 2, out);
+  k_norm2<<<g, kBlock, 0, c->stream>>>(v, len, e, c->partials, c->ticket + 2, out);
+  LZ_LAUNCH_CHECK();
+  return LZ_OK;
+}
+
+int lz_k_absmax_bits(lz_ctx* c, const double* v, uint64_t len, unsigned long long* out) {
+  k_absmax_bits<<<stream_grid(c, len), kBlock, 0, c->stream>>>(v, len, out);
   LZ_LAUNCH_CHECK();
   return LZ_OK;
 }
@@ -1823,7 +1848,7 @@ int lz_k_tridiag_expv_into(lz_ctx* c, uint32_t k, double* eigvals, double* eigve
   const size_t zt_bytes = (size_t)k * k * sizeof(double);
   const int in_smem = zt_bytes <= 180 * 1024;
   if (in_smem) LZ_CUDA(cudaFuncSetAttribute(k_tridiag_expv, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)zt_bytes));
-  k_tridiag_expv<<<1, kBlock, in_smem ? zt_bytes : 0, c->stream>>>(k, c->alpha, c->beta, c->scal + 2, eigvals, eigvecs, work, coef, status, in_smem,
+  k_tridiag_expv<<<1, kBlock, in_smem ? zt_bytes : 0, c->stream>>>(k, c->alpha, c->beta, c->scal + 2, c->x_exp, eigvals, eigvecs, work, coef, status, in_smem,
                                                                   c->matfun_kind, c->matfun_param, ls_in, ls_out);
   LZ_LAUNCH_CHECK();
   return LZ_OK;
@@ -1835,7 +1860,7 @@ int lz_k_tridiag_expv(lz_ctx* c, uint32_t k) {
 
 int lz_k_permute_in(lz_ctx* c, const double* x_orig, const double* norm2, uint64_t first, uint64_t count, double* dst) {
   unsigned g = stream_grid(c, count);
-  if (norm2) k_permute_in<<<g, kBlock, 0, c->stream>>>(x_orig, c->new2old, first, count, norm2, dst);
+  if (norm2) k_permute_in<<<g, kBlock, 0, c->stream>>>(x_orig, c->new2old, first, count, norm2, c->x_exp, dst);
   else k_permute_in_raw<<<g, kBlock, 0, c->stream>>>(x_orig, c->new2old, first, count, dst);
   LZ_LAUNCH_CHECK();
   return LZ_OK;
